@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our arm (one rank per GPU under torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K ...  the reference's CPU algorithm (oracle port, all host threads)
+  python bench.py ... --dump-outputs DIR                    also write what the last timed step computed to DIR/*.npy
 
 A "step" is ONE hot-path SQP iteration (SURVEY.md 8d) for every OCP of the batch, given the stage linearisations
 resident in HBM:  condense (PDIPM + contact/impact dynamics + SE(3) state-equation correction)  ->  backward Riccati
@@ -16,11 +17,14 @@ import argparse
 import ctypes
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -69,7 +73,30 @@ def parse():
     ap.add_argument("--batch", type=int, default=1024, help="OCP instances per GPU (BASELINE config 3: 1024)")
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                    "(float64, at most 64 MB; the inputs are the same on every run)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path: it needs --impl b200")
+    return args
+
+
+DUMP_BYTES = 60 * 10**6  # below 64 MB in all, .npy headers included
+DUMP_SEED = 0
+
+
+def dump_outputs(out_dir, sol, con, direction, steps):
+    """The records the timed iteration hands back -- updated solution, updated PDIPM records (slack | dual | residual), Newton
+    direction -- of a fixed, seeded sample of the batch's OCPs (as many as fit in DUMP_BYTES), and the primal / dual step sizes
+    of every OCP.  ocp_index lists the sampled OCPs."""
+    batch = sol.shape[0]
+    per_ocp = (sol[0].size + con[0].size + direction[0].size) * 8
+    n = min(batch, (DUMP_BYTES - steps.nbytes - batch * 8) // per_ocp)
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(batch, size=n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("solution", sol[idx]), ("constraint_data", con[idx]), ("direction", direction[idx]), ("step_sizes", steps),
+                    ("ocp_index", idx)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def build_problem(batch, seed):
@@ -212,14 +239,17 @@ def _oracle_runner(pr):
     os.environ.setdefault("OMP_DYNAMIC", "false")
     import oracle_lib
     lib = oracle_lib.load()
-    native = os.path.join(oracle_lib.ORACLE_DIR, "liboracle_native.so")
-    try:  # -march=native build of the same sources, made on this machine
-        # -B: always rebuilt here -- a copy that travelled from another machine was tuned for that machine's CPU
-        subprocess.run(["make", "-s", "-B", "-C", oracle_lib.ORACLE_DIR, "native"], check=True, stdout=subprocess.DEVNULL,
-                       stderr=subprocess.DEVNULL)
+    tmp = tempfile.mkdtemp(prefix="rbt_bench_")
+    native = os.path.join(tmp, "liboracle_native.so")
+    try:  # -march=native build of the same sources, made on this machine, in a temporary directory
+        # -B: always rebuilt -- the build must be tuned for this machine's CPU
+        subprocess.run(["make", "-s", "-B", "-C", oracle_lib.ORACLE_DIR, "native", f"NATIVE={native}"], check=True,
+                       stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
         lib = ct.CDLL(native)
     except Exception:
         pass
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)  # a loaded library stays mapped
     from robotoc_b200._lib import rbt_stage_ctrl
     from robotoc_b200.stage import rbt_constraint_table, rbt_stage_dims
     c_int, c_dbl, c_vp = ct.c_int, ct.c_double, ct.c_void_p
@@ -502,6 +532,8 @@ def main():
         assert err < 1e-8, f"rank {rank}: gathered step disagrees with the oracle ({err:.2e})"
     sol_dev = dms.getSolution()
     steps_dev = np.stack([dms.maxPrimalStepSize(), dms.maxDualStepSize()], axis=1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sol_dev, dms.getConstraintData(), d_local.cpu().numpy(), steps_dev)
 
     # ---- end-to-end arm: host (pinned) buffers through the one-call C-ABI entry point, H2D + D2H inside the timed region
     pin = lambda a: torch.from_numpy(a).pin_memory()  # noqa: E731

@@ -5,7 +5,8 @@
 The reference itself (Eigen3 + Pinocchio C++) cannot be built or imported in this image, and its test-suite holds no
 golden vectors (SURVEY.md section 4), so these fixtures pin the ORACLE (regression) and give the GPU tests a
 size-independent, file-based target; the oracle in turn is pinned by the identity tests (test_oracle_kkt.py,
-test_oracle_condense.py).  Inputs are regenerated from the seeds below by the tests; only outputs are stored.
+test_oracle_condense.py).  Inputs are regenerated from the seeds below by the tests; only outputs are stored, sampled by
+golden_io.
 """
 import ctypes
 import os
@@ -89,8 +90,18 @@ if __name__ == "__main__":
     kkt_c, steps, sol, con = iteration_case()
     kkt_cs, steps_s, sol_s, con_s = iteration_case(True)
     ukkt, usteps, usol, ucon = unconstr_iteration_case()
-    np.savez_compressed(os.path.join(HERE, "golden_r1.npz"), ric=ric, d=d, ric_sto=ric_s, d_sto=d_s, uric=uric, ud=ud,
-                        kkt_condensed=kkt_c, steps=steps, sol=sol, con=con,
-                        kkt_condensed_sto=kkt_cs, steps_sto=steps_s, sol_sto=sol_s, con_sto=con_s,
-                        ukkt_condensed=ukkt, usteps=usteps, usol=usol, ucon=ucon)
+    import golden_io
+    from robotoc_b200.unconstr_dms import UStageLayout, iiwa14_constraint_table
+    lib = oracle_lib.load()
+    K, UL = Layout(ANYMAL, getter=lib.orc_layout_get), ULayout(7, getter=lib.orc_ulayout_get)
+    table = anymal_constraint_table()
+    S = StageLayout(StageDims(ANYMAL, nf_max=12, n_contacts=4, n_box=table.n_box), getter=lib.orc_stage_layout_get)
+    US = UStageLayout(7, iiwa14_constraint_table().n_box, getter=lib.orc_ustage_layout_get)
+    data = dict(ric=ric, d=d, ric_sto=ric_s, d_sto=d_s, uric=uric, ud=ud, kkt_condensed=kkt_c, steps=steps, sol=sol, con=con,
+                kkt_condensed_sto=kkt_cs, steps_sto=steps_s, sol_sto=sol_s, con_sto=con_s,
+                ukkt_condensed=ukkt, usteps=usteps, usol=usol, ucon=ucon)
+    layouts = {"ric": (K, "r_"), "d": (K, "d_"), "uric": (UL, "r_"), "ud": (UL, "d_"), "kkt_condensed": (K, "k_"), "sol": (S, "s_"),
+               "con": (S, "c_"), "ukkt_condensed": (UL, "k_"), "usol": (US, "s_"), "ucon": (US, "c_")}
+    sections = {k: golden_io.sections(*layouts[k.replace("_sto", "")]) for k in data if k.replace("_sto", "") in layouts}
+    golden_io.save(os.path.join(HERE, "golden_r1.npz"), data, sections)
     print("wrote", os.path.join(HERE, "golden_r1.npz"), os.path.getsize(os.path.join(HERE, "golden_r1.npz")) // 1024, "KiB")

@@ -1,34 +1,25 @@
 """SURVEY.md 8f-2, first slice: the joint-limit half of Constraints::linearizeConstraints on the device
 (rbt_linearize_joint_limits: PDIPM residuals of the box rows + their dual terms in the gradients).
-CPU: the oracle against the reference's own JointPosition / Velocity / Torques Lower / Upper Limit classes (compiled unmodified,
-oracle/Makefile.ref) where /root/reference is available, and against a numpy statement of their formulas everywhere;
+CPU: the oracle against what the reference's own JointPosition / Velocity / Torques Lower / Upper Limit classes (compiled
+unmodified, oracle/Makefile.ref) computed on the same problems (tests/golden/golden_ref_stage_r2.npz, "jl_" keys, made by
+make_golden_ref_stage.py), and against a numpy statement of their formulas;
 GPU: the CUDA kernel against the oracle."""
 import ctypes
+import os
+import sys
 
 import numpy as np
 import pytest
 
 import oracle_lib
 from helpers import small_event_schedule, trot_schedule
-from robotoc_b200 import ANYMAL, StageDims, StageLayout, anymal_constraint_table
+from robotoc_b200 import ANYMAL, StageLayout
 from robotoc_b200.grid import IMPACT, TERMINAL
-from synth import make_stage_inputs
 
-
-def _problem(sched, batch, seed):
-    lib = oracle_lib.load()
-    table = anymal_constraint_table()
-    sd = StageDims(ANYMAL, nf_max=12, n_contacts=table.n_contacts, n_box=table.n_box)
-    S = StageLayout(sd, getter=lib.orc_stage_layout_get)
-    td, ev, ctrl = sched
-    lin, con, sol, dx0 = make_stage_inputs(sd, S, ctrl, batch, seed)
-    rng = np.random.default_rng(seed + 3)
-    lim = {0: 1.2, 1: 8.0, 3: 40.0}  # |q|, |v|, |u| limits of the order of ANYmal's URDF
-    bound = np.array([table.box[r].sign * lim[table.box[r].var] * rng.uniform(0.8, 1.2) for r in range(table.n_box)])
-    for k in (2, 4):  # the reference's velocity / torque limits are symmetric (joint_velocity_lower_limit.cpp: vmin = -vmax)
-        bound[k * 12:(k + 1) * 12] = -bound[(k + 1) * 12:(k + 2) * 12]
-    lib.orc_linearize_joint_limits_batch.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 4
-    return lib, table, sd, S, ctrl, lin, con, sol, bound
+HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.join(HERE, "golden"))
+import golden_io  # noqa: E402
+from make_golden_ref_stage import JOINT_LIMIT_PROBLEMS, joint_limit_problem  # noqa: E402
 
 
 def _oracle(lib, table, sd, ctrl, bound, sol, lin, con):
@@ -57,30 +48,22 @@ def _numpy(table, S, ctrl, bound, sol, lin, con):
     return l, c
 
 
-@pytest.mark.parametrize("which", ["small_sto", "trot"])
+@pytest.mark.parametrize("which", list(JOINT_LIMIT_PROBLEMS))
 def test_oracle_joint_limit_linearisation(which):
-    sched = {"small_sto": small_event_schedule(True), "trot": trot_schedule(40)}[which]
-    lib, table, sd, S, ctrl, lin, con, sol, bound = _problem(sched, 2, 81)
+    sched, batch, seed = JOINT_LIMIT_PROBLEMS[which]
+    lib, table, sd, S, ctrl, lin, con, sol, bound = joint_limit_problem(sched(), batch, seed)
     l_o, c_o = _oracle(lib, table, sd, ctrl, bound, sol, lin, con)
     l_n, c_n = _numpy(table, S, ctrl, bound, sol, lin, con)
     np.testing.assert_allclose(l_o, l_n, rtol=1e-15, atol=1e-15)
     np.testing.assert_allclose(c_o, c_n, rtol=1e-15, atol=1e-15)
     assert np.abs(l_o - lin).max() > 0.01 and np.abs(c_o - con).max() > 0.1   # it did something
     assert np.array_equal(c_o[:, 0, S.c_res:S.c_res + 48], con[:, 0, S.c_res:S.c_res + 48])  # stage 0: position / velocity rows gated
-    import ref_lib
-    if not ref_lib.available():
-        return
-    rl = ref_lib.load()
-    rl.ref_linearize_joint_limits.argtypes = [ctypes.c_void_p] * 7
-    csd = sd.c()
-    P = oracle_lib.ptr
-    for b in range(lin.shape[0]):
-        for i, ct in enumerate(ctrl):
-            l_r, c_r = np.ascontiguousarray(lin[b, i]), np.ascontiguousarray(con[b, i])
-            assert rl.ref_linearize_joint_limits(ctypes.byref(csd), ctypes.byref(table), ctypes.byref(ct), P(bound),
-                                                 P(np.ascontiguousarray(sol[b, i])), P(l_r), P(c_r)) == 0
-            np.testing.assert_allclose(l_o[b, i], l_r, rtol=1e-14, atol=1e-14, err_msg=f"gradient, grid {i}")
-            np.testing.assert_allclose(c_o[b, i], c_r, rtol=1e-14, atol=1e-14, err_msg=f"residual, grid {i}")
+    # the reference's classes, stored as what they changed: every entry they left alone, a sample of the ones they set
+    G = golden_io.load(os.path.join(HERE, "golden", "golden_ref_stage_r2.npz"))
+    for got, inp, delta in ((l_o, lin, G[f"jl_{which}_dlin"]), (c_o, con, G[f"jl_{which}_dcon"])):
+        m = golden_io.finite(delta)
+        assert m.any() and np.any(delta[m] != 0.0)
+        np.testing.assert_allclose(got[m], (inp + delta)[m], rtol=1e-14, atol=1e-14)
 
 
 @pytest.mark.gpu
@@ -88,7 +71,7 @@ def test_oracle_joint_limit_linearisation(which):
 def test_cuda_joint_limit_linearisation_matches_the_oracle(which, batch):
     from robotoc_b200 import DirectMultipleShooting, RiccatiRecursion
     sched = {"small_sto": small_event_schedule(True), "trot": trot_schedule(40)}[which]
-    lib, table, sd, S, ctrl, lin, con, sol, bound = _problem(sched, batch, 82)
+    lib, table, sd, S, ctrl, lin, con, sol, bound = joint_limit_problem(sched, batch, 82)
     S = StageLayout(sd)
     rr = RiccatiRecursion(ANYMAL, len(ctrl), batch)
     rr.setTimeDiscretization(ctrl)

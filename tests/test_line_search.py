@@ -1,8 +1,11 @@
 """SURVEY.md 8f-3: batched trial step sizes + the filter acceptance loop of robotoc::LineSearch.
-CPU: the oracle's filter loop against the reference's own LineSearchFilter class (compiled unmodified into oracle/_ref) over
-     many consecutive line searches; the oracle's trial solutions against its own update at the same step size.
+CPU: the oracle's filter loop against what the reference's own LineSearchFilter class (compiled unmodified, oracle/Makefile.ref)
+     accepted over many consecutive line searches (tests/golden/golden_ref_seeds.npz, made by make_golden_ref.py); the
+     oracle's trial solutions against its own update at the same step size.
 GPU: the CUDA path against the oracle."""
 import ctypes
+import os
+import sys
 
 import numpy as np
 import pytest
@@ -13,6 +16,11 @@ from iteration_check import oracle_iteration
 from robotoc_b200 import ANYMAL, Layout, StageDims, StageLayout, anymal_constraint_table
 from robotoc_b200.grid import IMPACT, TERMINAL
 from synth import make_stage_inputs
+
+HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.join(HERE, "golden"))
+import golden_io  # noqa: E402
+import make_golden_ref as mg  # noqa: E402
 
 T_Q, T_V, T_A, T_U, T_F, T_STRIDE = 0, 20, 38, 56, 68, 80
 CAP = 16
@@ -36,29 +44,18 @@ def _filter_oracle(lib, steps, cost0, viol0, cost, barrier, viol, filt, nfilt, r
 
 
 def test_oracle_filter_loop_equals_the_reference_line_search_filter():
-    import ref_lib
-    if not ref_lib.available():
-        pytest.skip("oracle/_ref not built and /root/reference not present")
-    lib, ref = _orc(), ref_lib.load()
-    ref.ref_filter_line_search.argtypes = [ctypes.c_int, ctypes.c_int] + [ctypes.c_double] * 4 + [ctypes.c_void_p] * 7
-    rng = np.random.default_rng(3)
-    rounds, n_trials = 40, 8
-    for case in range(20):
-        amax = rng.uniform(0.05, 1.0, size=rounds)
-        trend = np.linspace(10.0, 1.0, rounds)[:, None]  # costs drift down like a converging solver; violations shrink
-        cost = trend + rng.normal(0, 0.5, size=(rounds, n_trials))
-        viol = np.abs(trend * 0.1 + rng.normal(0, 0.05, size=(rounds, n_trials)))
-        cost0, viol0 = cost[:, 0] + 0.1, viol[:, 0] + 0.01
-        step_r, k_r = np.zeros(rounds), np.zeros(rounds, dtype=np.int32)
-        P = oracle_lib.ptr
-        ref.ref_filter_line_search(rounds, n_trials, 0.75, 0.05, 0.005, 0.005, P(amax), P(cost0), P(viol0), P(np.ascontiguousarray(cost)),
-                                   P(np.ascontiguousarray(viol)), P(step_r), k_r.ctypes.data_as(ctypes.c_void_p))
+    lib = _orc()
+    G = golden_io.load(os.path.join(HERE, "golden", "golden_ref_seeds.npz"))
+    f = mg.FILTER
+    for case, (amax, cost0, viol0, cost, viol) in enumerate(mg.filter_cases()):
+        step_r, k_r = G["filter_step"][case], G["filter_k"][case]
         # the oracle: one "OCP" (batch 1) whose filter persists across the rounds
         filt, nfilt = np.zeros((1, 2 * CAP)), np.zeros(1, dtype=np.int32)
-        for r in range(rounds):
+        for r in range(f["rounds"]):
             steps = np.array([[amax[r], 1.0]])
             st, kk = _filter_oracle(lib, steps, cost0[r:r + 1].copy(), viol0[r:r + 1].copy(), np.ascontiguousarray(cost[r][:, None]),
-                                    np.zeros((n_trials, 1)), np.ascontiguousarray(viol[r][:, None]), filt, nfilt)
+                                    np.zeros((f["n_trials"], 1)), np.ascontiguousarray(viol[r][:, None]), filt, nfilt, rate=f["rate"],
+                                    min_step=f["min_step"], cr=f["cost_reduction"], vr=f["violation_reduction"])
             assert kk[0] == k_r[r] and st[0] == step_r[r], (case, r)
         assert nfilt[0] <= CAP
 
