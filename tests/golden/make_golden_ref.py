@@ -2,7 +2,7 @@
 src/riccati/*.cpp + src/core/split_*.cpp compiled unmodified (oracle/Makefile.ref, Eigen / Robot stand-ins of oracle/shim).
 Only runs where a checkout of the reference is available (ROBOTOC_REFERENCE, see oracle/Makefile.ref):
 
-    python tests/golden/make_golden_ref.py
+    python tests/golden/make_golden_ref.py [FILE.npz ...]     # default: every file below
 
 Inputs are regenerated from the seeds below by the tests (tests/synth.py); only the reference's outputs are stored, sampled
 by golden_io.  golden_ref_r2.npz:
@@ -11,7 +11,7 @@ by golden_io.  golden_ref_r2.npz:
     N=40, jump STO N=80).
 golden_ref_seeds.npz:
   - "field_*": every Riccati / direction record and the KKT blocks the recursion mutates, batch 3, on further seeds
-    (FIELD_CASES, UNCONSTR_FIELD_CASES);
+    (FIELD_CASES, UNCONSTR_FIELD_CASES; the crawl schedules' records are in golden_ref_seeds_crawl.npz);
   - "filter_*": accepted step size and trial index of the reference's LineSearchFilter over consecutive line searches
     (filter_cases()).
 tests/test_golden_ref.py and tests/test_line_search.py check the oracle (CPU) and the CUDA path (-m gpu) against these files.
@@ -26,7 +26,7 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
-from helpers import jump_sto_schedule, small_event_schedule, trot_schedule  # noqa: E402
+from helpers import crawl_schedule, jump_sto_schedule, small_event_schedule, trot_schedule  # noqa: E402
 from robotoc_b200 import ANYMAL  # noqa: E402
 from synth import make_kkt, make_unconstr_kkt  # noqa: E402
 
@@ -39,7 +39,8 @@ CASES = {  # name -> (schedule factory, seed, batch, store full records?)
     "jump_sto_n80": (lambda: jump_sto_schedule(80), 204, 1, False),
 }
 UNCONSTR = dict(nv=7, N=20, dt=0.05, seed=205, batch=2)
-FIELD_CASES = {"small": 31, "small_sto": 32, "trot_n40": 33, "jump_sto_n80": 34}  # name -> seed, batch 3
+FIELD_CASES = {"small": 31, "small_sto": 32, "trot_n40": 33, "jump_sto_n80": 34,  # name -> seed, batch 3
+               "crawl_small": 35, "crawl_small_sto": 36}
 UNCONSTR_FIELD_CASES = ((20, 0.05, 41), (50, 0.02, 42))                           # (N, dt, seed), batch 3
 FILTER = dict(cases=20, rounds=40, n_trials=8, rate=0.75, min_step=0.05, cost_reduction=0.005, violation_reduction=0.005)
 
@@ -82,8 +83,19 @@ def unconstr_inputs(UL):
     return make_unconstr_kkt(u["nv"], UL, u["N"], u["batch"], u["seed"])
 
 
+def field_schedule(name):
+    if name.startswith("crawl_small"):
+        return crawl_schedule("crawl_small", sto=name.endswith("_sto"))
+    return CASES[name][0]()
+
+
+def field_path(name):
+    """The file that holds the "field_<name>_*" records."""
+    return os.path.join(HERE, "golden_ref_seeds_crawl.npz" if name.startswith("crawl") else "golden_ref_seeds.npz")
+
+
 def field_inputs(name, seed, L):
-    td, ev, ctrl = CASES[name][0]()
+    td, ev, ctrl = field_schedule(name)
     kkt, dx0 = make_kkt(ANYMAL, L, ctrl, batch=3, seed=seed)
     return ctrl, kkt, dx0
 
@@ -107,24 +119,34 @@ if __name__ == "__main__":
     import oracle_lib
     import ref_lib
     from robotoc_b200 import Layout, ULayout
+    only = set(sys.argv[1:])
+
+    def wanted(path):
+        return not only or os.path.basename(path) in only
+
     lib = oracle_lib.load()
     L = Layout(ANYMAL, getter=lib.orc_layout_get)
-    out = {}
-    for name in CASES:
-        ctrl, kkt, dx0, full = inputs(name, L)
-        kk, ric, d = ref_lib.riccati_batch(ANYMAL, L, ctrl, kkt, dx0)
-        out[name + "_ric"] = ric if full else trim(L, ric)
-        out[name + "_dir"] = d
     UL = ULayout(7, getter=lib.orc_ulayout_get)
-    kkt, dx0 = unconstr_inputs(UL)
-    kk, ric, d = ref_lib.unconstr_batch(7, UL, UNCONSTR["N"], UNCONSTR["dt"], kkt, dx0)
-    out["unconstr_ric"], out["unconstr_dir"] = ric, d
     path = os.path.join(HERE, "golden_ref_r2.npz")
-    golden_io.save(path, out, record_sections(L, UL, out))
-    out = {}
+    if wanted(path):
+        out = {}
+        for name in CASES:
+            ctrl, kkt, dx0, full = inputs(name, L)
+            kk, ric, d = ref_lib.riccati_batch(ANYMAL, L, ctrl, kkt, dx0)
+            out[name + "_ric"] = ric if full else trim(L, ric)
+            out[name + "_dir"] = d
+        kkt, dx0 = unconstr_inputs(UL)
+        kk, ric, d = ref_lib.unconstr_batch(7, UL, UNCONSTR["N"], UNCONSTR["dt"], kkt, dx0)
+        out["unconstr_ric"], out["unconstr_dir"] = ric, d
+        golden_io.save(path, out, record_sections(L, UL, out))
+        print("wrote", path, os.path.getsize(path) // 1024, "KiB")
+    files = {}  # path -> arrays
     for name, seed in FIELD_CASES.items():
         ctrl, kkt, dx0 = field_inputs(name, seed, L)
+        out = files.setdefault(field_path(name), {})
         out[f"field_{name}_kkt"], out[f"field_{name}_ric"], out[f"field_{name}_dir"] = ref_lib.riccati_batch(ANYMAL, L, ctrl, kkt, dx0)
+    path_seeds = field_path("small")
+    out = files[path_seeds]
     for N, dt, seed in UNCONSTR_FIELD_CASES:
         kkt, dx0 = make_unconstr_kkt(7, UL, N, 3, seed)
         out[f"field_unconstr{N}_kkt"], out[f"field_unconstr{N}_ric"], out[f"field_unconstr{N}_dir"] = ref_lib.unconstr_batch(7, UL, N, dt, kkt, dx0)
@@ -139,7 +161,8 @@ if __name__ == "__main__":
                                    P(steps[case]), k.ctypes.data_as(ctypes.c_void_p))
         ks[case] = k
     out["filter_step"], out["filter_k"] = steps, ks
-    path_seeds = os.path.join(HERE, "golden_ref_seeds.npz")
-    golden_io.save(path_seeds, out, record_sections(L, UL, out), block=64)  # batch 3 on long horizons: a thinner sample
-    print("wrote", path, os.path.getsize(path) // 1024, "KiB,", path_seeds, os.path.getsize(path_seeds) // 1024, "KiB;",
-          ref.ref_version().decode())
+    for path, out in files.items():
+        if wanted(path):
+            golden_io.save(path, out, record_sections(L, UL, out), block=64)  # batch 3 on long horizons: a thinner sample
+            print("wrote", path, os.path.getsize(path) // 1024, "KiB")
+    print(ref.ref_version().decode())

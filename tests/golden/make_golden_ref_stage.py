@@ -2,7 +2,7 @@
 (tests/ref_lib.reference_iteration: the reference's src/dynamics, src/constraints, src/core and src/riccati compiled unmodified,
 oracle/Makefile.ref).  Only runs where a checkout of the reference is available (ROBOTOC_REFERENCE, see oracle/Makefile.ref):
 
-    python tests/golden/make_golden_ref_stage.py
+    python tests/golden/make_golden_ref_stage.py [FILE.npz ...]     # default: every file below
 
 Stored (sampled by golden_io):
   - one FULL iteration on the small event schedule with switching-time optimisation (Intermediate, Lift,
@@ -22,7 +22,7 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
-from helpers import small_event_schedule, trot_schedule  # noqa: E402
+from helpers import crawl_schedule, small_event_schedule, trot_schedule  # noqa: E402
 from robotoc_b200 import ANYMAL  # noqa: E402
 from robotoc_b200.stage import StageDims, anymal_constraint_table  # noqa: E402
 from synth import make_stage_inputs  # noqa: E402
@@ -31,7 +31,8 @@ import golden_io  # noqa: E402
 
 SEED, BATCH = 301, 1
 KEYS = ("kkt", "cc_cond", "ric", "d", "cc_exp", "xd_exp", "steps", "d_upd", "xd_upd", "cc_upd", "ex_upd", "perf_stage")
-SEED_CASES = {"small": 311, "small_sto": 312, "trot": 313, "small_icone": 314, "small_sto_icone": 315}  # name -> seed, batch 1
+SEED_CASES = {"small": 311, "small_sto": 312, "trot": 313, "small_icone": 314, "small_sto_icone": 315,  # name -> seed, batch 1
+              "crawl_small": 317, "crawl_small_sto": 318, "crawl_small_icone": 319}
 SEED_KEYS = ("kkt", "cc_cond", "ric", "cc_exp", "xd_exp", "steps", "d_upd", "xd_upd", "cc_upd", "ex_upd")
 # the records are compared section by section at every grid point: every grid point keeps the short sections (dx, du, lx, lu,
 # e_lup, e_r, ...) whole and at least 36 entries of each longer one
@@ -57,8 +58,11 @@ def seed_problem(which, seed, S_getter=None, K_getter=None):
     table = anymal_constraint_table(impact_friction_cone=icone)
     sd = StageDims(ANYMAL, nf_max=12, n_contacts=table.n_contacts, n_box=table.n_box)
     S, K = StageLayout(sd, getter=S_getter), Layout(ANYMAL, getter=K_getter)
-    td, ev, ctrl = {"small": small_event_schedule(False), "small_sto": small_event_schedule(True), "trot": trot_schedule(40),
-                    "small_icone": small_event_schedule(False), "small_sto_icone": small_event_schedule(True)}[which]
+    td, ev, ctrl = {"small": lambda: small_event_schedule(False), "small_sto": lambda: small_event_schedule(True),
+                    "trot": lambda: trot_schedule(40), "small_icone": lambda: small_event_schedule(False),
+                    "small_sto_icone": lambda: small_event_schedule(True), "crawl_small": lambda: crawl_schedule("crawl_small"),
+                    "crawl_small_sto": lambda: crawl_schedule("crawl_small", sto=True),
+                    "crawl_small_icone": lambda: crawl_schedule("crawl_small")}[which]()
     lin, con, sol, dx0 = make_stage_inputs(sd, S, ctrl, 1, seed, impact_cones=icone)
     return table, sd, S, K, ctrl, lin, con, sol, dx0
 
@@ -120,37 +124,45 @@ if __name__ == "__main__":
 
     import oracle_lib
     import ref_lib
+    only = set(sys.argv[1:])
+
+    def wanted(path):
+        return not only or os.path.basename(path) in only
+
     lib = oracle_lib.load()
-    table, sd, S, K, ctrl, lin, con, sol, dx0 = problem(lib.orc_stage_layout_get, lib.orc_layout_get)
-    out = ref_lib.reference_iteration(sd, S, K, table, ctrl, lin, con, dx0)
-    data = {k: out[k] for k in KEYS}
-    table, sd, S, K, ctrl, lin, con, sol, dx0 = problem(lib.orc_stage_layout_get, lib.orc_layout_get, impact_cones=True)
-    out = ref_lib.reference_iteration(sd, S, K, table, ctrl, lin, con, dx0)
-    data.update({"ic_" + k: out[k] for k in KEYS})
-    for impact_cones in (False, True):
-        table, sd, S, K, ctrl, lin, con, sol, dx0 = perf_trot_problem(impact_cones, lib.orc_stage_layout_get, lib.orc_layout_get)
-        data[f"perf_trot_{int(impact_cones)}"] = ref_lib.reference_iteration(sd, S, K, table, ctrl, lin, con, dx0)["perf_stage"]
-    rl = ref_lib.load()
-    rl.ref_linearize_joint_limits.argtypes = [ctypes.c_void_p] * 7
-    P = oracle_lib.ptr
-    for which, (sched, batch, seed) in JOINT_LIMIT_PROBLEMS.items():
-        lib_, table, sd, S, ctrl, lin, con, sol, bound = joint_limit_problem(sched(), batch, seed)
-        l_r, c_r = lin.copy(), con.copy()
-        csd = sd.c()
-        for b in range(batch):
-            for i, ct in enumerate(ctrl):
-                lb, cb = lin[b, i].copy(), con[b, i].copy()
-                assert rl.ref_linearize_joint_limits(ctypes.byref(csd), ctypes.byref(table), ctypes.byref(ct), P(bound),
-                                                     P(np.ascontiguousarray(sol[b, i])), P(lb), P(cb)) == 0
-                l_r[b, i], c_r[b, i] = lb, cb
-        data[f"jl_{which}_dlin"], data[f"jl_{which}_dcon"] = l_r - lin, c_r - con
     path = os.path.join(HERE, "golden_ref_stage_r2.npz")
-    golden_io.save(path, data, record_sections(S, K, data), **PER_GRID_POINT)
-    print("wrote", path, os.path.getsize(path) // 1024, "KiB")
+    if wanted(path):
+        table, sd, S, K, ctrl, lin, con, sol, dx0 = problem(lib.orc_stage_layout_get, lib.orc_layout_get)
+        out = ref_lib.reference_iteration(sd, S, K, table, ctrl, lin, con, dx0)
+        data = {k: out[k] for k in KEYS}
+        table, sd, S, K, ctrl, lin, con, sol, dx0 = problem(lib.orc_stage_layout_get, lib.orc_layout_get, impact_cones=True)
+        out = ref_lib.reference_iteration(sd, S, K, table, ctrl, lin, con, dx0)
+        data.update({"ic_" + k: out[k] for k in KEYS})
+        for impact_cones in (False, True):
+            table, sd, S, K, ctrl, lin, con, sol, dx0 = perf_trot_problem(impact_cones, lib.orc_stage_layout_get, lib.orc_layout_get)
+            data[f"perf_trot_{int(impact_cones)}"] = ref_lib.reference_iteration(sd, S, K, table, ctrl, lin, con, dx0)["perf_stage"]
+        rl = ref_lib.load()
+        rl.ref_linearize_joint_limits.argtypes = [ctypes.c_void_p] * 7
+        P = oracle_lib.ptr
+        for which, (sched, batch, seed) in JOINT_LIMIT_PROBLEMS.items():
+            lib_, table, sd, S, ctrl, lin, con, sol, bound = joint_limit_problem(sched(), batch, seed)
+            l_r, c_r = lin.copy(), con.copy()
+            csd = sd.c()
+            for b in range(batch):
+                for i, ct in enumerate(ctrl):
+                    lb, cb = lin[b, i].copy(), con[b, i].copy()
+                    assert rl.ref_linearize_joint_limits(ctypes.byref(csd), ctypes.byref(table), ctypes.byref(ct), P(bound),
+                                                         P(np.ascontiguousarray(sol[b, i])), P(lb), P(cb)) == 0
+                    l_r[b, i], c_r[b, i] = lb, cb
+            data[f"jl_{which}_dlin"], data[f"jl_{which}_dcon"] = l_r - lin, c_r - con
+        golden_io.save(path, data, record_sections(S, K, data), **PER_GRID_POINT)
+        print("wrote", path, os.path.getsize(path) // 1024, "KiB")
     for which, seed in SEED_CASES.items():
+        path = seed_path(which)
+        if not wanted(path):
+            continue
         table, sd, S, K, ctrl, lin, con, sol, dx0 = seed_problem(which, seed, lib.orc_stage_layout_get, lib.orc_layout_get)
         out = ref_lib.reference_iteration(sd, S, K, table, ctrl, lin, con, dx0)
         data = {k: out[k] for k in SEED_KEYS}
-        path = seed_path(which)
         golden_io.save(path, data, record_sections(S, K, data), **dict(PER_GRID_POINT, block=1 << 30))  # min_keep entries only
         print("wrote", path, os.path.getsize(path) // 1024, "KiB")

@@ -3,7 +3,7 @@ import numpy as np
 
 from robotoc_b200 import ANYMAL, Layout
 from robotoc_b200.grid import IMPACT, LIFT, TERMINAL
-from schedule_fixture import (ContactEvents, TimeDiscretization, stage_ctrl_array, anymal_trot_events,
+from schedule_fixture import (ContactEvents, TimeDiscretization, stage_ctrl_array, anymal_crawl_events, anymal_trot_events,
                               anymal_jump_sto_events)
 from synth import make_kkt, mat
 
@@ -26,6 +26,20 @@ def trot_schedule(N=40):
 def jump_sto_schedule(N=80):
     ev = anymal_jump_sto_events()
     td = TimeDiscretization(1.7, N).discretize(ev, 0.0, sto=True)
+    return td, ev, stage_ctrl_array(td, ev)
+
+
+CRAWL_SIZES = {"crawl_full": dict(cycle=2, swing=0.5, ds=0.04),   # examples/anymal/crawl.cpp itself: N = 210, 219 grid points
+               "crawl_small": dict(cycle=1, swing=0.1, ds=0.04)}  # every event kind and contact dimension: N = 26, 31 grid points
+
+
+def crawl_schedule(size="crawl_small", sto=False, dt=0.02):
+    """ANYmal crawl (schedule_fixture.anymal_crawl_events): phases with three feet in contact (nf = 9), single-foot impacts
+    (nf = 3 on the Impact stage, ns = 3 on the switching-constraint stage before it).  N = T / dt as crawl.cpp computes it."""
+    p = CRAWL_SIZES[size]
+    ev = anymal_crawl_events(p["cycle"], p["swing"], p["ds"], sto=sto)
+    T = p["ds"] + p["cycle"] * (4 * p["swing"] + 2 * p["ds"])
+    td = TimeDiscretization(T, int(T / dt)).discretize(ev, 0.0, sto=sto)
     return td, ev, stage_ctrl_array(td, ev)
 
 

@@ -262,6 +262,24 @@ def anymal_trot_events() -> ContactEvents:
     return ev
 
 
+def anymal_crawl_events(cycle: int = 2, swing: float = 0.5, ds: float = 0.04, sto: bool = False) -> ContactEvents:
+    """Contact schedule of /root/reference/examples/anymal/crawl.cpp:43-46,161-229: one foot in the air at a time, per cycle
+    stand(12) -lift RH-> (9) -RH closes, RF opens-> (9) -RF closes-> stand -lift LH-> (9) -LH closes, LF opens-> (9) -LF closes->
+    stand.  Every impact is a single foot (impact dimf 3, so the switching constraint before it has ns = 3), and two of them
+    lift another foot at the same instant.  T = t0 + cycle * (4 swing + 2 ds) with t0 = ds; sto: every event's time is optimised."""
+    ev = ContactEvents(phase_dimf=[12], phase_mask=[0b1111])
+    t0 = ds
+    for k in range(cycle):
+        t1 = t0 + k * (2 * ds + 4 * swing)
+        ev.push_back(False, t1, 9, sto=sto, post_mask=0b0111)                                           # RH lifts
+        ev.push_back(True, t1 + swing, 9, impact_dimf=3, sto=sto, post_mask=0b1011, impact_mask=0b1000)  # RH closes, RF opens
+        ev.push_back(True, t1 + 2 * swing, 12, impact_dimf=3, sto=sto, post_mask=0b1111, impact_mask=0b0100)  # RF closes
+        ev.push_back(False, t1 + ds + 2 * swing, 9, sto=sto, post_mask=0b1101)                          # LH lifts
+        ev.push_back(True, t1 + ds + 3 * swing, 9, impact_dimf=3, sto=sto, post_mask=0b1110, impact_mask=0b0010)  # LH closes, LF opens
+        ev.push_back(True, t1 + ds + 4 * swing, 12, impact_dimf=3, sto=sto, post_mask=0b1111, impact_mask=0b0001)  # LF closes
+    return ev
+
+
 def anymal_jump_sto_events() -> ContactEvents:
     """Contact schedule of /root/reference/examples/anymal/jump_sto.cpp:42-48,131-140:
     stand(12) -lift@0.4 (sto)-> flying(0) -impact@0.9 (sto)-> stand; T=1.7."""

@@ -54,20 +54,19 @@ def seeds():
     return golden_io.load(os.path.join(HERE, "golden", "golden_ref_seeds.npz"))
 
 
-@pytest.mark.parametrize("name,seed", list(mg.FIELD_CASES.items()))
-def test_oracle_equals_live_reference_every_field(seeds, name, seed):
-    """Every field of every Riccati / direction record and the mutated KKT blocks (F, H, G, lu'), batch 3, fresh seeds."""
-    lib = oracle_lib.load()
-    L = Layout(ANYMAL, getter=lib.orc_layout_get)
-    ctrl, kkt, dx0 = mg.field_inputs(name, seed, L)
-    kk_o, ric_o, d_o, info = oracle_lib.riccati_batch(ANYMAL, L, ctrl, kkt, dx0)
-    assert info == 0
-    kk_r, ric_r, d_r = (seeds[f"field_{name}_{k}"] for k in ("kkt", "ric", "dir"))
+def field_fixture(name):
+    """(kkt, ric, dir) of FIELD_CASES[name] as the reference computed them."""
+    g = golden_io.load(mg.field_path(name))
+    return tuple(g[f"field_{name}_{k}"] for k in ("kkt", "ric", "dir"))
+
+
+def assert_every_field(L, ctrl, kk, ric, d, kk_r, ric_r, d_r, tol=TOL):
+    """Every field of the Riccati records, the direction records and the mutated KKT blocks, over the entries the fixture holds."""
     fields = sorted((getattr(L, f), f) for f in ("r_P r_s r_K r_k r_M r_m r_Psi r_Phi r_T r_W r_psix r_psiu r_phix r_phiu r_mt "
                                                   "r_mtn r_sc r_dtsdx r_stosc").split())
     ends = [o for o, _ in fields[1:]] + [L.r_stosc + 2]
     for (o, f), e in zip(fields, ends):
-        a, b = ric_o[..., o:e], ric_r[..., o:e]
+        a, b = ric[..., o:e], ric_r[..., o:e]
         m = golden_io.finite(b)
         assert m.all() or np.any(b[m]), f"{f}: the fixture holds none of the field's non-zeros"
         a, b = a[m], b[m]
@@ -78,9 +77,21 @@ def test_oracle_equals_live_reference_every_field(seeds, name, seed):
             # ns == nu: W = -(Ginv - SDG^T DG) phi_u with an analytically zero matrix -> pure cancellation noise in both codes
             assert np.max(np.abs(a - b)) < 1e-9 * np.nanmax(np.abs(ric_r[..., L.r_T:L.r_T + ANYMAL.nu])), f
         else:
-            assert np.max(np.abs(a - b)) < TOL * scale, f"{f}: {np.max(np.abs(a - b)) / scale:.2e}"
-    assert _rel(d_o, d_r) < TOL
-    assert _rel(kk_o, kk_r) < TOL  # in-place mutation semantics: Qxx, Qxu, Quu, lu <- F (- K^T G K), H, G, lu'
+            assert np.max(np.abs(a - b)) < tol * scale, f"{f}: {np.max(np.abs(a - b)) / scale:.2e}"
+    assert _rel(d, d_r) < tol
+    if kk is not None:
+        assert _rel(kk, kk_r) < tol  # in-place mutation semantics: Qxx, Qxu, Quu, lu <- F (- K^T G K), H, G, lu'
+
+
+@pytest.mark.parametrize("name,seed", list(mg.FIELD_CASES.items()))
+def test_oracle_equals_live_reference_every_field(name, seed):
+    """Every field of every Riccati / direction record and the mutated KKT blocks (F, H, G, lu'), batch 3, fresh seeds."""
+    lib = oracle_lib.load()
+    L = Layout(ANYMAL, getter=lib.orc_layout_get)
+    ctrl, kkt, dx0 = mg.field_inputs(name, seed, L)
+    kk_o, ric_o, d_o, info = oracle_lib.riccati_batch(ANYMAL, L, ctrl, kkt, dx0)
+    assert info == 0
+    assert_every_field(L, ctrl, kk_o, ric_o, d_o, *field_fixture(name))
 
 
 def test_oracle_equals_live_reference_unconstr(seeds):

@@ -58,13 +58,27 @@ def _cmp_rows(name, S, c, icone, f, got, ref):
         _cmp(name, got[:, o:o + S.nc], ref[:, o:o + S.nc])
 
 
-def _run(ctrl, batch, seed, reserve=0, impact_cones=False):
+def poison_inactive_contact_rows(S, ctrl, lin):
+    """A copy of the linearization records with NaN in the rows nf..nf_max-1 of every contact Jacobian J: rows no kernel may
+    use (a record reused from a phase with more contacts, or left by the wire format, which never writes them)."""
+    out = lin.copy()
+    for i, c in enumerate(ctrl):
+        if c.type != TERMINAL:
+            J = out[:, i, S.l_J:S.l_J + S.nfm * S.nv].reshape(-1, S.nv, S.nfm)  # [batch, col, row]
+            J[:, :, c.nf:] = np.nan
+    return out
+
+
+def _run(ctrl, batch, seed, reserve=0, impact_cones=False, poison=False):
+    """poison: the device gets the records with NaN in the inactive rows of J (poison_inactive_contact_rows)."""
     lib = oracle_lib.load()
     table = anymal_constraint_table(impact_friction_cone=impact_cones)
     sd = StageDims(ANYMAL, nf_max=12, n_contacts=table.n_contacts, n_box=table.n_box)
     S, K = StageLayout(sd), Layout(ANYMAL)
     lin, con, sol, dx0 = make_stage_inputs(sd, S, ctrl, batch, seed, impact_cones=impact_cones)
     ref = _oracle_iteration(lib, sd, S, K, table, ctrl, lin, con, sol, dx0)
+    if poison:
+        lin = poison_inactive_contact_rows(S, ctrl, lin)
     rr = RiccatiRecursion(ANYMAL, len(ctrl) + reserve, batch)  # reserve: the reference sizes for N + 1 + reserved events
     rr.setTimeDiscretization(ctrl)
     dms = DirectMultipleShooting(rr, sd, table)
