@@ -4,6 +4,7 @@
 #include <cstring>
 #include <cstdint>
 #include <cstdlib>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -11,7 +12,6 @@
 #include <dlfcn.h>
 
 #include <algorithm>
-#include <cstdlib>
 
 #include "../../include/robotoc_b200.h"
 #include "riccati_backward.cuh"
@@ -37,10 +37,60 @@ struct Err {
     }                                                                                         \
   } while (0)
 
-template <class K>
-int set_smem(K kernel, size_t bytes) {
-  return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) == cudaSuccess ? 0 : 1;
+// Device memory, streams and events owned by a handle: released when the handle is deleted (after rbt_destroy has made
+// the handle's device current).
+struct CudaRelease {
+  void operator()(void* p) const { cudaFree(p); }
+  void operator()(CUstream_st* s) const { cudaStreamDestroy(s); }
+  void operator()(CUevent_st* e) const { cudaEventDestroy(e); }
+};
+template <class T>
+using Owned = std::unique_ptr<T, CudaRelease>;
+
+template <class T>
+cudaError_t dev_alloc(Owned<T>& p, size_t n) {
+  p.reset();
+  T* q = nullptr;
+  const cudaError_t e = cudaMalloc(&q, n * sizeof(T));
+  p.reset(q);
+  return e;
 }
+
+// The public buffers of a handle, indexed by RBT_BUF_*.  `ptr` is what the kernels use: the handle's own allocation, or
+// a caller's buffer bound with rbt_bind_buffer (never freed by the handle).
+struct BufTable {
+  struct Entry {
+    Owned<double> own;
+    double* ptr = nullptr;
+    int per_row = 0;        // doubles per row
+    bool per_grid = false;  // a row per grid point of every OCP (else one row per OCP)
+  };
+  Entry e[RBT_BUF_PERF + 1];
+  long long batch = 0;
+  int n_grid_max = 0;
+
+  static bool valid(int which) { return which >= 0 && which <= RBT_BUF_PERF; }
+  double* operator[](int which) const { return valid(which) ? e[which].ptr : nullptr; }
+  long long doubles(int which, int n_grid) const {
+    if (!valid(which) || !e[which].own) return -1;
+    return batch * (e[which].per_grid ? n_grid : 1) * e[which].per_row;
+  }
+  // the handle's own allocation, zeroed
+  cudaError_t alloc(int which, int per_row, bool per_grid) {
+    Entry& x = e[which];
+    x.per_row = per_row;
+    x.per_grid = per_grid;
+    const size_t n = size_t(batch) * (per_grid ? n_grid_max : 1) * per_row;
+    const cudaError_t err = dev_alloc(x.own, n);
+    x.ptr = x.own.get();
+    return err != cudaSuccess ? err : cudaMemset(x.ptr, 0, n * 8);
+  }
+};
+
+// A contiguous range [b0, b0 + nb) of the batch that a launch or a copy works on.
+struct Win {
+  int b0, nb;
+};
 
 }  // namespace
 
@@ -49,84 +99,63 @@ struct rbt_handle {
   rbt_layout L;
   int n_grid_max = 0, n_grid = 0, batch = 0, device = 0;
   double max_dts0 = 0.1;
-  rbt_stage_ctrl* d_ctrl = nullptr;
+  Owned<rbt_stage_ctrl> d_ctrl;
   std::vector<rbt_stage_ctrl> ctrl;  // host copy
-  double *d_kkt = nullptr, *d_ric = nullptr, *d_fact = nullptr, *d_dir = nullptr, *d_dx0 = nullptr;
-  double* own[12] = {};  // the handle's own allocation of a buffer that the caller re-bound (freed in destroy)
-  int* d_info = nullptr;
-  int* d_arrivals = nullptr;  // per-SM CTA arrival counters (CTA de-phasing in the backward kernel)
-  int* d_struct = nullptr;    // [0]: 1 = every Fxx of the KKT buffer has the mechanical structure (see rbt_set_fxx_structure)
+  BufTable buf;
+  Owned<int> d_info;
+  Owned<int> d_struct;  // [0]: 1 = every Fxx of the KKT buffer has the mechanical structure (see rbt_set_fxx_structure)
   int fxx_mode = RBT_FXX_AUTO;
   bool kkt_from_condense = false;  // the KKT records were just written by rbt_condense: structure holds by construction
-  int stagger_ns = 0;
-  long long* d_timeline = nullptr;  // bring-up instrumentation (RBT_TIMELINE_CTA)
   // stage layer
   bool stage_ready = false;
   bool keep_info = false;  // condense's Cholesky flags survive the following backward launch
   rbt_stage_dims sdims;
   rbt_stage_layout S;
   rbt_constraint_table table;
-  double *d_lin = nullptr, *d_con = nullptr, *d_ex = nullptr, *d_sol = nullptr, *d_xd = nullptr, *d_steps = nullptr,
-         *d_ones = nullptr;
-  double *d_stage_perf = nullptr, *d_perf = nullptr, *d_x0in = nullptr;  // eval_kernels.cuh
+  Owned<double> d_ones, d_stage_perf, d_x0in;  // eval_kernels.cuh
   // line search (line_search_kernels.cuh): trial buffers sized on first use, filter state per OCP
   int ls_trials = 0;
-  double *d_ls_alphas = nullptr, *d_ls_trial = nullptr, *d_ls_stage_barrier = nullptr, *d_ls_barrier = nullptr;
-  double *d_ls_in = nullptr, *d_ls_filt = nullptr, *d_ls_step = nullptr;
-  int *d_ls_nfilt = nullptr, *d_ls_k = nullptr;
-  double* d_step_pack = nullptr;  // packed Newton step of this rank (rbt_allgather_step), allocated on first use
-  int timeline_cta = -1;
+  Owned<double> d_ls_alphas, d_ls_trial, d_ls_stage_barrier, d_ls_barrier, d_ls_in, d_ls_filt, d_ls_step;
+  Owned<int> d_ls_nfilt, d_ls_k;
+  Owned<double> d_step_pack;  // packed Newton step of this rank (rbt_allgather_step), allocated on first use
   long long launches = 0;
-  // batch window [cb0, cb0 + cnb) the launch helpers work on (cnb == 0: the whole batch); used by rbt_iteration_host to
-  // pipeline uploads, kernels and downloads over chunks of the batch
-  int cb0 = 0, cnb = 0;
-  double* d_wire = nullptr;  // packed host wire records (rbt_iteration_host_wire), allocated on first use
-  int* d_tgt = nullptr;           // box rows per PDIPM target (stage_kernels.cuh: StageParams::tgt)
-  double* d_bound = nullptr;      // joint limits per box row (rbt_set_joint_limits)
-  double* d_res_stage = nullptr;  // rbt_iteration_host_resident: compact residuals in, compact slack|dual out
-  double* d_sd_stage = nullptr;
+  Owned<double> d_wire;       // packed host wire records (rbt_iteration_host_wire), allocated on first use
+  Owned<int> d_tgt;           // box rows per PDIPM target (stage_kernels.cuh: StageParams::tgt)
+  Owned<double> d_bound;      // joint limits per box row (rbt_set_joint_limits)
+  Owned<double> d_res_stage;  // rbt_iteration_host_resident: compact residuals in, compact slack|dual out
+  Owned<double> d_sd_stage;
   std::vector<rbt_wire_layout> Wv;   // per grid point (the wire record of a grid point depends on its control word)
-  rbt_wire_layout* d_W = nullptr;
+  Owned<rbt_wire_layout> d_W;
   long long w_ocp = 0;               // doubles of one OCP's concatenated wire records
   int cost_structure = RBT_COST_GENERAL;  // what the host's wire records hold (rbt_set_wire_cost_structure)
   bool wire_dirty = true;                 // per-grid-point wire layouts on the device are stale (schedule / cost structure changed)
   bool attr_bwd = false, attr_fwd = false, attr_cond = false;  // MaxDynamicSharedMemorySize set on THIS handle's device
   cudaEvent_t ev_condense_mid = nullptr;  // caller-owned event recorded between the two kernels of rbt_condense (timing)
-  cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
-  std::vector<cudaEvent_t> ev;
+  Owned<CUstream_st> s_h2d, s_d2h;
+  std::vector<Owned<CUevent_st>> ev;
   std::string err;
 };
-
-static inline int win_b0(const rbt_handle* h) { return h->cnb ? h->cb0 : 0; }
-static inline int win_nb(const rbt_handle* h) { return h->cnb ? h->cnb : h->batch; }
 
 struct rbt_uhandle {
   int nv = 0, N = 0, batch = 0, device = 0;
   double dt = 0;
   rbt_ulayout L;
-  double *d_kkt = nullptr, *d_ric = nullptr, *d_fact = nullptr, *d_dir = nullptr, *d_dx0 = nullptr;
-  int* d_info = nullptr;
+  BufTable buf;
+  Owned<int> d_info;
   // stage layer
   bool stage_ready = false;
   rbt_ustage_layout S;
   rbt_constraint_table table;
-  double *d_lin = nullptr, *d_con = nullptr, *d_ex = nullptr, *d_sol = nullptr, *d_xd = nullptr, *d_steps = nullptr,
-         *d_ones = nullptr;
+  Owned<double> d_ones;
   long long launches = 0;
   std::string err;
 };
 
 // ---- compiled instances ------------------------------------------------------------------------------------------
-// ANYmal (floating base + 4 point contacts): nv=18, nu=12, max_dimf=12     src/robot/robot.cpp:33-60
-#define RBT_INSTANCES(X) X(18, 12, 12)
-
-static bool instance_supported(const rbt_dims& d) {
-#define X(NV, NU, NS) \
-  if (d.nv == NV && d.nu == NU && d.ns_max == NS) return true;
-  RBT_INSTANCES(X)
-#undef X
-  return false;
-}
+// constrained: ANYmal (floating base + 4 point contacts), nv=18, nu=12, max_dimf=12     src/robot/robot.cpp:33-60
+constexpr int INST_NV = 18, INST_NU = 12, INST_NS = 12;
+// unconstrained: iiwa14, nv=7
+constexpr int UINST_NV = 7;
 
 // All functions below are declared extern "C" in include/robotoc_b200.h; the definitions inherit that linkage.
 
@@ -163,40 +192,29 @@ int rbt_device_info(int device, int* sm, int* n_sm, char* name, int name_len) {
 
 int rbt_create(const rbt_dims* dims, int n_grid_max, int batch, int device, rbt_handle** out) {
   if (!dims || !out || n_grid_max < 2 || batch < 1 || dims->nv < 1 || dims->nu < 1 || dims->ns_max < 0) return RBT_ERR_ARG;
-  if (!instance_supported(*dims)) return RBT_ERR_ARG;
+  if (dims->nv != INST_NV || dims->nu != INST_NU || dims->ns_max != INST_NS) return RBT_ERR_ARG;
   rbt_handle* h = new rbt_handle();
   h->dims = *dims;
   rbt_make_layout(dims, &h->L);
   h->n_grid_max = n_grid_max;
   h->batch = batch;
   h->device = device;
+  h->buf.batch = batch;
+  h->buf.n_grid_max = n_grid_max;
   *out = h;
   RBT_CUDA(h, cudaSetDevice(device));
-  const size_t per = size_t(batch) * n_grid_max;
-  RBT_CUDA(h, cudaMalloc(&h->d_ctrl, sizeof(rbt_stage_ctrl) * n_grid_max));
-  RBT_CUDA(h, cudaMalloc(&h->d_kkt, per * h->L.k_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_ric, per * h->L.r_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_fact, per * h->L.f_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_dir, per * h->L.d_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_dx0, size_t(batch) * h->L.nx * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_info, size_t(batch) * sizeof(int)));
-  RBT_CUDA(h, cudaMalloc(&h->d_arrivals, 1024 * sizeof(int)));
-  RBT_CUDA(h, cudaMalloc(&h->d_struct, 4 * sizeof(int)));
-  RBT_CUDA(h, cudaMemset(h->d_struct, 0, 4 * sizeof(int)));
-  h->stagger_ns = getenv("RBT_STAGGER_NS") ? atoi(getenv("RBT_STAGGER_NS")) : 0;
-  if (getenv("RBT_TIMELINE_CTA")) {
-    h->timeline_cta = atoi(getenv("RBT_TIMELINE_CTA"));
-    RBT_CUDA(h, cudaMalloc(&h->d_timeline, size_t(n_grid_max) * 32 * sizeof(long long)));
-    RBT_CUDA(h, cudaMemset(h->d_timeline, 0, size_t(n_grid_max) * 32 * sizeof(long long)));
-  }
-  RBT_CUDA(h, cudaMemset(h->d_ric, 0, per * h->L.r_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_fact, 0, per * h->L.f_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_dir, 0, per * h->L.d_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_info, 0, size_t(batch) * sizeof(int)));
+  RBT_CUDA(h, dev_alloc(h->d_ctrl, n_grid_max));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_KKT, h->L.k_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_RIC, h->L.r_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_FACT, h->L.f_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_DIR, h->L.d_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_DX0, h->L.nx, false));
+  RBT_CUDA(h, dev_alloc(h->d_info, batch));
+  RBT_CUDA(h, dev_alloc(h->d_struct, 4));
+  RBT_CUDA(h, cudaMemset(h->d_struct.get(), 0, 4 * sizeof(int)));
+  RBT_CUDA(h, cudaMemset(h->d_info.get(), 0, size_t(batch) * sizeof(int)));
   return RBT_OK;
 }
-
-static double** buf_slot(rbt_handle* h, int which);
 
 // The stage kernels are compiled for nf_max / n_contacts of the constraint table: every grid of the schedule must fit.
 static int check_contacts(rbt_handle* h, const rbt_stage_ctrl* ctrl, int n_grid) {
@@ -210,36 +228,8 @@ static int check_contacts(rbt_handle* h, const rbt_stage_ctrl* ctrl, int n_grid)
 }
 
 int rbt_destroy(rbt_handle* h) {
-  if (h) {
-    cudaFree(h->d_wire);
-    cudaFree(h->d_W);
-    cudaFree(h->d_tgt);
-    cudaFree(h->d_bound);
-    cudaFree(h->d_res_stage);
-    cudaFree(h->d_sd_stage);
-    if (h->s_h2d) cudaStreamDestroy(h->s_h2d);
-    if (h->s_d2h) cudaStreamDestroy(h->s_d2h);
-    for (cudaEvent_t e : h->ev) cudaEventDestroy(e);
-  }
   if (!h) return RBT_ERR_ARG;
   cudaSetDevice(h->device);
-  cudaFree(h->d_ctrl);
-  for (int q = 0; q <= RBT_BUF_XDIR; ++q) {
-    double** slot = buf_slot(h, q);
-    if (slot) cudaFree(h->own[q] ? h->own[q] : *slot);  // never free a caller-owned buffer
-  }
-  cudaFree(h->d_info);
-  cudaFree(h->d_arrivals);
-  cudaFree(h->d_struct);
-  cudaFree(h->d_timeline);
-  cudaFree(h->d_steps);
-  cudaFree(h->d_ones);
-  cudaFree(h->d_step_pack);
-  cudaFree(h->d_ls_alphas); cudaFree(h->d_ls_trial); cudaFree(h->d_ls_stage_barrier); cudaFree(h->d_ls_barrier);
-  cudaFree(h->d_ls_in); cudaFree(h->d_ls_filt); cudaFree(h->d_ls_step); cudaFree(h->d_ls_nfilt); cudaFree(h->d_ls_k);
-  cudaFree(h->d_stage_perf);
-  cudaFree(h->d_perf);
-  cudaFree(h->d_x0in);
   delete h;
   return RBT_OK;
 }
@@ -281,10 +271,10 @@ int rbt_set_schedule(rbt_handle* h, const rbt_stage_ctrl* ctrl, int n_grid, doub
   }
   if (check_contacts(h, ctrl, n_grid) != RBT_OK) return RBT_ERR_ARG;
   RBT_CUDA(h, cudaSetDevice(h->device));
-  RBT_CUDA(h, cudaMemcpy(h->d_ctrl, ctrl, sizeof(rbt_stage_ctrl) * n_grid, cudaMemcpyHostToDevice));
+  RBT_CUDA(h, cudaMemcpy(h->d_ctrl.get(), ctrl, sizeof(rbt_stage_ctrl) * n_grid, cudaMemcpyHostToDevice));
   // stage-conditional outputs (M, STO terms, policies) must not leak from a previous schedule
-  RBT_CUDA(h, cudaMemset(h->d_ric, 0, size_t(h->batch) * n_grid * h->L.r_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_dir, 0, size_t(h->batch) * n_grid * h->L.d_stride * 8));
+  RBT_CUDA(h, cudaMemset(h->buf[RBT_BUF_RIC], 0, size_t(h->buf.doubles(RBT_BUF_RIC, n_grid)) * 8));
+  RBT_CUDA(h, cudaMemset(h->buf[RBT_BUF_DIR], 0, size_t(h->buf.doubles(RBT_BUF_DIR, n_grid)) * 8));
   h->n_grid = n_grid;
   h->max_dts0 = max_dts0;
   h->ctrl.assign(ctrl, ctrl + n_grid);
@@ -292,80 +282,26 @@ int rbt_set_schedule(rbt_handle* h, const rbt_stage_ctrl* ctrl, int n_grid, doub
   return RBT_OK;
 }
 
-static double* buf_ptr(rbt_handle* h, int which) {
-  switch (which) {
-    case RBT_BUF_KKT: return h->d_kkt;
-    case RBT_BUF_RIC: return h->d_ric;
-    case RBT_BUF_FACT: return h->d_fact;
-    case RBT_BUF_DIR: return h->d_dir;
-    case RBT_BUF_DX0: return h->d_dx0;
-    case RBT_BUF_LIN: return h->d_lin;
-    case RBT_BUF_CON: return h->d_con;
-    case RBT_BUF_EXP: return h->d_ex;
-    case RBT_BUF_SOL: return h->d_sol;
-    case RBT_BUF_XDIR: return h->d_xd;
-    case RBT_BUF_STEPS: return h->d_steps;
-    case RBT_BUF_PERF: return h->d_perf;
-    default: return nullptr;
-  }
-}
-
 long long rbt_buf_doubles(rbt_handle* h, int which) {
-  if (!h) return -1;
-  const long long per = (long long)h->batch * h->n_grid;
-  if (which >= RBT_BUF_LIN && !h->stage_ready) return -1;
-  switch (which) {
-    case RBT_BUF_LIN: return per * h->S.l_stride;
-    case RBT_BUF_CON: return per * h->S.c_stride;
-    case RBT_BUF_EXP: return per * h->S.e_stride;
-    case RBT_BUF_SOL: return per * h->S.s_stride;
-    case RBT_BUF_XDIR: return per * h->S.x_stride;
-    case RBT_BUF_STEPS: return 2LL * h->batch;
-    case RBT_BUF_PERF: return 8LL * h->batch;
-    case RBT_BUF_KKT: return per * h->L.k_stride;
-    case RBT_BUF_RIC: return per * h->L.r_stride;
-    case RBT_BUF_FACT: return per * h->L.f_stride;
-    case RBT_BUF_DIR: return per * h->L.d_stride;
-    case RBT_BUF_DX0: return (long long)h->batch * h->L.nx;
-    default: return -1;
-  }
+  if (!h || (which >= RBT_BUF_LIN && !h->stage_ready)) return -1;
+  return h->buf.doubles(which, h->n_grid);
 }
 
-double* rbt_dev_ptr(rbt_handle* h, int which) { return h ? buf_ptr(h, which) : nullptr; }
-
-static double** buf_slot(rbt_handle* h, int which) {
-  switch (which) {
-    case RBT_BUF_KKT: return &h->d_kkt;
-    case RBT_BUF_RIC: return &h->d_ric;
-    case RBT_BUF_FACT: return &h->d_fact;
-    case RBT_BUF_DIR: return &h->d_dir;
-    case RBT_BUF_DX0: return &h->d_dx0;
-    case RBT_BUF_LIN: return &h->d_lin;
-    case RBT_BUF_CON: return &h->d_con;
-    case RBT_BUF_EXP: return &h->d_ex;
-    case RBT_BUF_SOL: return &h->d_sol;
-    case RBT_BUF_XDIR: return &h->d_xd;
-    default: return nullptr;
-  }
-}
+double* rbt_dev_ptr(rbt_handle* h, int which) { return h ? h->buf[which] : nullptr; }
 
 int rbt_bind_buffer(rbt_handle* h, int which, double* dev) {
   if (!h) return RBT_ERR_ARG;
-  double** slot = buf_slot(h, which);
-  if (!slot || (which >= RBT_BUF_LIN && !h->stage_ready)) return RBT_ERR_ARG;
-  if (!h->own[which]) h->own[which] = *slot;  // remember the handle's own allocation the first time it is replaced
-  double* q = dev ? dev : h->own[which];
+  // STEPS, PERF and INFO stay the handle's own
+  if (which < 0 || which > RBT_BUF_XDIR || which == RBT_BUF_INFO || (which >= RBT_BUF_LIN && !h->stage_ready)) return RBT_ERR_ARG;
+  double* q = dev ? dev : h->buf.e[which].own.get();
   if ((reinterpret_cast<uintptr_t>(q) & 15u) != 0) {
     h->err = "[rbt_bind_buffer] invalid argument: device buffer must be 16-byte aligned";
     return RBT_ERR_ARG;
   }
-  *slot = q;
+  h->buf.e[which].ptr = q;
   return RBT_OK;
 }
 
-static long long stage_xfer(rbt_handle* h, int which, bool up, const double* host_c, double* host_m, int b0, int nb,
-                            cudaStream_t st, bool do_copy, int* rc_out);
-enum { RBT_XFER_WIRE = 100, RBT_XFER_SWITCHING = 101, RBT_XFER_RES = 102, RBT_XFER_SD = 103 };
 // the STO section of the linearization records is read on switching-time stages only (riccati_backward.cuh: cs.sto)
 static int ctrl_has_sto(const rbt_stage_ctrl* ctrl, int n_grid) {
   for (int i = 0; i < n_grid; ++i)
@@ -388,52 +324,147 @@ static long long make_wire_layouts(const rbt_stage_layout& S, const rbt_stage_ct
 static int ensure_wire_layouts(rbt_handle* h) {  // rebuilt only when the schedule or the cost structure changed
   if (!h->wire_dirty && h->d_W) return RBT_OK;
   h->w_ocp = make_wire_layouts(h->S, h->ctrl.data(), h->n_grid, h->cost_structure, h->Wv);
-  if (!h->d_W) RBT_CUDA(h, cudaMalloc(&h->d_W, size_t(h->n_grid_max) * sizeof(rbt_wire_layout)));
-  RBT_CUDA(h, cudaMemcpy(h->d_W, h->Wv.data(), size_t(h->n_grid) * sizeof(rbt_wire_layout), cudaMemcpyHostToDevice));
+  if (!h->d_W) RBT_CUDA(h, dev_alloc(h->d_W, h->n_grid_max));
+  RBT_CUDA(h, cudaMemcpy(h->d_W.get(), h->Wv.data(), size_t(h->n_grid) * sizeof(rbt_wire_layout), cudaMemcpyHostToDevice));
   h->wire_dirty = false;
   return RBT_OK;
 }
 
-// KKT upload plan: one strided copy of the core section [Fxx|Fvu|Fx|lx|lu|Qxx|Qxu|Quu] of every record (record padding and
-// unused switching/STO sections never cross PCIe), plus one strided copy per stage that carries extras.
-static long long kkt_upload(rbt_handle* h, const double* host, cudaStream_t st, bool do_copy, int* rc_out) {
-  const rbt_layout& L = h->L;
-  const size_t pitch = size_t(L.k_stride) * 8;
-  int n_extra = 0;
-  for (const auto& c : h->ctrl) n_extra += (c.ns > 0 || c.sto) ? 1 : 0;
-  const bool wide = n_extra * 2 > h->n_grid;  // most stages carry extras (STO horizons): copy core+extras in one go
-  const size_t width = size_t(wide ? L.k_core_size + L.k_extra_size : L.k_core_size) * 8;
-  const size_t rows = size_t(h->batch) * h->n_grid;
-  long long bytes = (long long)(width * rows);
-  if (do_copy && cudaMemcpy2DAsync(h->d_kkt, pitch, host, pitch, width, rows, cudaMemcpyHostToDevice, st) != cudaSuccess) {
-    *rc_out = RBT_ERR_CUDA;
-    return 0;
+// ---- host <-> device transfers -----------------------------------------------------------------------------------
+// The host arrays a transfer plan reads or writes.  Each has the layout of the device buffer it is copied to or from.
+enum HostArg { A_KKT, A_LIN, A_WIRE, A_RES, A_CON, A_SOL, A_DX0, A_SOL_OUT, A_CON_OUT, A_STEPS_OUT, N_HOST_ARGS };
+// What crosses PCIe in rbt_iteration_host (DENSE), rbt_iteration_host_wire (WIRE) and rbt_iteration_host_resident (RESIDENT).
+enum HostMode { DENSE = 0, WIRE = 1, RESIDENT = 2 };
+
+namespace {
+// One copy: `rows` rows of `width` doubles, `pitch` doubles apart, starting `off` doubles into the device buffer `dev` and
+// into the host array `arg`.
+struct Copy {
+  cudaMemcpyKind kind;
+  int arg;
+  double* dev;
+  size_t off, pitch, width, rows;
+};
+
+// Builds the copies of the batch window `w`.  Only what the kernels read or what persists crosses PCIe: record padding
+// never does, the switching-constraint and STO sections only for the stages that carry them.
+struct Plan {
+  const rbt_handle* h;
+  Win w;
+  std::vector<Copy> c;
+
+  // the section [off, off + width) of the records (`stride` doubles each) of every grid point of the window
+  void records(cudaMemcpyKind k, int arg, double* dev, size_t stride, size_t off, size_t width) {
+    const size_t g = size_t(h->n_grid);
+    c.push_back({k, arg, dev, size_t(w.b0) * g * stride + off, stride, width, size_t(w.nb) * g});
   }
-  if (!wide) {
-    const size_t opitch = pitch * h->n_grid;
-    for (int i = 0; i < h->n_grid; ++i) {
-      const rbt_stage_ctrl& c = h->ctrl[i];
-      if (!(c.ns > 0 || c.sto)) continue;
-      const size_t off = size_t(i) * L.k_stride + L.k_Phix;
-      bytes += (long long)(size_t(L.k_extra_size) * 8 * h->batch);
-      if (do_copy && cudaMemcpy2DAsync(h->d_kkt + off, opitch, host + off, opitch, size_t(L.k_extra_size) * 8, h->batch,
-                                       cudaMemcpyHostToDevice, st) != cudaSuccess) {
-        *rc_out = RBT_ERR_CUDA;
-        return 0;
-      }
-    }
+  // n doubles per OCP of the window
+  void per_ocp(cudaMemcpyKind k, int arg, double* dev, size_t n) {
+    c.push_back({k, arg, dev, size_t(w.b0) * n, n, n, size_t(w.nb)});
   }
+  // the section [off, off + width) of the records of grid point i of every OCP of the window
+  void grid_point(int arg, double* dev, size_t stride, int i, size_t off, size_t width) {
+    const size_t pitch = size_t(h->n_grid) * stride;
+    c.push_back({cudaMemcpyHostToDevice, arg, dev, size_t(w.b0) * pitch + size_t(i) * stride + off, pitch, width, size_t(w.nb)});
+  }
+  // KKT records: the core section [Fxx|Fvu|Fx|lx|lu|Qxx|Qxu|Quu] of every record, plus the extras of the stages that carry
+  // them (switching constraint, STO)
+  void kkt() {
+    const rbt_layout& L = h->L;
+    int n_extra = 0;
+    for (const auto& q : h->ctrl) n_extra += (q.ns > 0 || q.sto) ? 1 : 0;
+    const bool wide = n_extra * 2 > h->n_grid;  // most stages carry extras (STO horizons): copy core+extras in one go
+    records(cudaMemcpyHostToDevice, A_KKT, h->buf[RBT_BUF_KKT], L.k_stride, 0, wide ? L.k_core_size + L.k_extra_size : L.k_core_size);
+    if (wide) return;
+    for (int i = 0; i < h->n_grid; ++i)
+      if (h->ctrl[i].ns > 0 || h->ctrl[i].sto) grid_point(A_KKT, h->buf[RBT_BUF_KKT], L.k_stride, i, L.k_Phix, L.k_extra_size);
+  }
+  // the switching-constraint sections (Phix, Phia, p, Phit) of the linearization records
+  void switching() {
+    const rbt_stage_layout& S = h->S;
+    for (int i = 0; i < h->n_grid; ++i)
+      if (h->ctrl[i].ns > 0 && h->ctrl[i].type != RBT_IMPACT)
+        grid_point(A_LIN, h->buf[RBT_BUF_LIN], S.l_stride, i, S.l_Phix, S.l_ha - S.l_Phix);
+  }
+  void lin() {
+    const rbt_stage_layout& S = h->S;
+    records(cudaMemcpyHostToDevice, A_LIN, h->buf[RBT_BUF_LIN], S.l_stride, 0, S.l_Phix);  // M .. se3
+    records(cudaMemcpyHostToDevice, A_LIN, h->buf[RBT_BUF_LIN], S.l_stride, S.l_ha,        // ha .. dgdf
+            size_t(S.l_dgdf) + ((15 * S.ncon + 1) & ~1) - S.l_ha);
+    switching();
+  }
+  // PDIPM records: slack | dual | residual go up, slack | dual come back
+  void con(cudaMemcpyKind k, int arg) {
+    const rbt_stage_layout& S = h->S;
+    records(k, arg, h->buf[RBT_BUF_CON], S.c_stride, S.c_slack, size_t(k == cudaMemcpyHostToDevice ? 3 : 2) * S.ncp);
+  }
+  // whole records incl. the few padding doubles: ONE contiguous DMA instead of a strided 2-D copy of 1.4 KB rows (the copy
+  // engine spends as long per row as on ~4 KB of payload)
+  void sol(cudaMemcpyKind k, int arg) { records(k, arg, h->buf[RBT_BUF_SOL], h->S.s_stride, 0, h->S.s_stride); }
+  void dx0() { per_ocp(cudaMemcpyHostToDevice, A_DX0, h->buf[RBT_BUF_DX0], h->L.nx); }
+};
+
+// rbt_upload(which) of the whole batch
+std::vector<Copy> upload_plan(const rbt_handle* h, int which) {
+  Plan p{h, {0, h->batch}, {}};
+  if (which == RBT_BUF_KKT) p.kkt();
+  if (which == RBT_BUF_LIN) p.lin();
+  if (which == RBT_BUF_CON) p.con(cudaMemcpyHostToDevice, A_CON);
+  if (which == RBT_BUF_SOL) p.sol(cudaMemcpyHostToDevice, A_SOL);
+  if (which == RBT_BUF_DX0) p.dx0();
+  return p.c;
+}
+
+// one rbt_iteration_host* call on the batch window w (the wire modes need ensure_wire_layouts first)
+std::vector<Copy> host_plan(const rbt_handle* h, HostMode mode, Win w) {
+  const rbt_stage_layout& S = h->S;
+  Plan p{h, w, {}};
+  if (mode == DENSE) {
+    p.lin();
+  } else {
+    p.per_ocp(cudaMemcpyHostToDevice, A_WIRE, h->d_wire.get(), h->w_ocp);  // packed wire records
+    p.switching();
+  }
+  if (mode == RESIDENT) {  // compact PDIPM residuals [batch][n_grid][ncp] (unpack_wire_kernel scatters them into c_res)
+    p.records(cudaMemcpyHostToDevice, A_RES, h->d_res_stage.get(), S.ncp, 0, S.ncp);
+  } else {
+    p.con(cudaMemcpyHostToDevice, A_CON);
+    p.sol(cudaMemcpyHostToDevice, A_SOL);
+  }
+  p.dx0();
+  p.sol(cudaMemcpyDeviceToHost, A_SOL_OUT);
+  if (mode == RESIDENT)  // compact slack | dual [batch][n_grid][2 ncp] (packed by pack_slack_dual_kernel)
+    p.records(cudaMemcpyDeviceToHost, A_CON_OUT, h->d_sd_stage.get(), 2 * S.ncp, 0, 2 * S.ncp);
+  else
+    p.con(cudaMemcpyDeviceToHost, A_CON_OUT);
+  p.per_ocp(cudaMemcpyDeviceToHost, A_STEPS_OUT, h->buf[RBT_BUF_STEPS], 2);
+  return p.c;
+}
+
+long long plan_bytes(const std::vector<Copy>& plan, cudaMemcpyKind k) {
+  long long bytes = 0;
+  for (const Copy& c : plan)
+    if (c.kind == k) bytes += (long long)(c.width * c.rows * 8);
   return bytes;
 }
 
+int issue(rbt_handle* h, const Copy& c, const double* host_in, double* host_out, cudaStream_t st) {
+  const bool up = c.kind == cudaMemcpyHostToDevice;
+  void* dst = up ? static_cast<void*>(c.dev + c.off) : static_cast<void*>(host_out + c.off);
+  const void* src = up ? static_cast<const void*>(host_in + c.off) : static_cast<const void*>(c.dev + c.off);
+  if (c.pitch == c.width)  // contiguous: one linear DMA
+    RBT_CUDA(h, cudaMemcpyAsync(dst, src, c.width * c.rows * 8, c.kind, st));
+  else
+    RBT_CUDA(h, cudaMemcpy2DAsync(dst, c.pitch * 8, src, c.pitch * 8, c.width * 8, c.rows, c.kind, st));
+  return RBT_OK;
+}
+}  // namespace
+
 long long rbt_upload_bytes(rbt_handle* h, int which) {
   if (!h || h->n_grid == 0) return -1;
-  int rc = RBT_OK;
-  if (which == RBT_BUF_DX0) return rbt_buf_doubles(h, which) * 8;
-  if (which == RBT_BUF_LIN || which == RBT_BUF_CON || which == RBT_BUF_SOL)
-    return h->stage_ready ? stage_xfer(h, which, true, nullptr, nullptr, 0, h->batch, nullptr, false, &rc) : -1;
-  if (which != RBT_BUF_KKT) return -1;
-  return kkt_upload(h, nullptr, nullptr, false, &rc);
+  const bool stage_buf = which == RBT_BUF_LIN || which == RBT_BUF_CON || which == RBT_BUF_SOL;
+  if (!(which == RBT_BUF_KKT || which == RBT_BUF_DX0 || (stage_buf && h->stage_ready))) return -1;
+  return plan_bytes(upload_plan(h, which), cudaMemcpyHostToDevice);
 }
 
 int rbt_upload(rbt_handle* h, int which, const double* host, void* stream) {
@@ -443,35 +474,17 @@ int rbt_upload(rbt_handle* h, int which, const double* host, void* stream) {
   if (which >= RBT_BUF_LIN && !h->stage_ready) return RBT_ERR_STATE;
   if (h->n_grid == 0) return RBT_ERR_STATE;
   RBT_CUDA(h, cudaSetDevice(h->device));
-  if (which == RBT_BUF_KKT) {
-    int rc = RBT_OK;
-    h->kkt_from_condense = false;
-    kkt_upload(h, host, (cudaStream_t)stream, true, &rc);
-    if (rc != RBT_OK) {
-      h->err = std::string("rbt_upload(KKT): ") + cudaGetErrorString(cudaGetLastError());
-      return rc;
-    }
-    return RBT_OK;
-  }
-  if (which != RBT_BUF_DX0) {  // trimmed strided copies (see stage_xfer)
-    int rc = RBT_OK;
-    stage_xfer(h, which, true, host, nullptr, 0, h->batch, (cudaStream_t)stream, true, &rc);
-    if (rc != RBT_OK) {
-      h->err = std::string("rbt_upload: ") + cudaGetErrorString(cudaGetLastError());
-      return rc;
-    }
-    return RBT_OK;
-  }
-  RBT_CUDA(h, cudaMemcpyAsync(buf_ptr(h, which), host, size_t(rbt_buf_doubles(h, which)) * 8, cudaMemcpyHostToDevice,
-                              (cudaStream_t)stream));
+  if (which == RBT_BUF_KKT) h->kkt_from_condense = false;
+  for (const Copy& c : upload_plan(h, which))
+    if (int rc = issue(h, c, host, nullptr, (cudaStream_t)stream)) return rc;
   return RBT_OK;
 }
 
 int rbt_download(rbt_handle* h, int which, double* host, void* stream) {
-  if (!h || !host || !buf_ptr(h, which)) return RBT_ERR_ARG;
+  if (!h || !host || !h->buf[which]) return RBT_ERR_ARG;
   if (h->n_grid == 0) return RBT_ERR_STATE;
   RBT_CUDA(h, cudaSetDevice(h->device));
-  RBT_CUDA(h, cudaMemcpyAsync(host, buf_ptr(h, which), size_t(rbt_buf_doubles(h, which)) * 8, cudaMemcpyDeviceToHost,
+  RBT_CUDA(h, cudaMemcpyAsync(host, h->buf[which], size_t(rbt_buf_doubles(h, which)) * 8, cudaMemcpyDeviceToHost,
                               (cudaStream_t)stream));
   return RBT_OK;
 }
@@ -479,7 +492,7 @@ int rbt_download(rbt_handle* h, int which, double* host, void* stream) {
 int rbt_download_info(rbt_handle* h, int* host_flags, void* stream) {
   if (!h || !host_flags) return RBT_ERR_ARG;
   RBT_CUDA(h, cudaSetDevice(h->device));
-  RBT_CUDA(h, cudaMemcpyAsync(host_flags, h->d_info, size_t(h->batch) * sizeof(int), cudaMemcpyDeviceToHost,
+  RBT_CUDA(h, cudaMemcpyAsync(host_flags, h->d_info.get(), size_t(h->batch) * sizeof(int), cudaMemcpyDeviceToHost,
                               (cudaStream_t)stream));
   return RBT_OK;
 }
@@ -488,7 +501,7 @@ int rbt_check_info(rbt_handle* h, int* first_bad, void* stream) {
   if (!h) return RBT_ERR_ARG;
   RBT_CUDA(h, cudaSetDevice(h->device));
   std::vector<int> flags(size_t(h->batch), 0);
-  RBT_CUDA(h, cudaMemcpyAsync(flags.data(), h->d_info, flags.size() * sizeof(int), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+  RBT_CUDA(h, cudaMemcpyAsync(flags.data(), h->d_info.get(), flags.size() * sizeof(int), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
   RBT_CUDA(h, cudaStreamSynchronize((cudaStream_t)stream));
   if (first_bad) *first_bad = -1;
   for (int b = 0; b < h->batch; ++b)
@@ -501,16 +514,15 @@ int rbt_check_info(rbt_handle* h, int* first_bad, void* stream) {
   return RBT_OK;
 }
 
-template <int NV, int NU, int NS>
-static int launch_backward(rbt_handle* h, int write_fact, cudaStream_t st) {
+static int launch_backward(rbt_handle* h, Win w, int write_fact, cudaStream_t st) {
   constexpr int NP = 6;
-  using C = rbt::BwdCfg<NV, NU, NS, NP>;
+  using C = rbt::BwdCfg<INST_NV, INST_NU, INST_NS, NP>;
   if (C::STAGE != h->L.k_stage_size || C::EXTRA != h->L.k_extra_size) {
     h->err = "internal: shared-memory staging size does not match rbt_layout";
     return RBT_ERR_STATE;
   }
-  auto kern_s = rbt::riccati_backward_kernel<NV, NU, NS, NP, true>;   // Fqq = I, Fqv = dt I outside the floating-base blocks
-  auto kern_g = rbt::riccati_backward_kernel<NV, NU, NS, NP, false>;  // any Fxx
+  auto kern_s = rbt::riccati_backward_kernel<INST_NV, INST_NU, INST_NS, NP, true>;   // Fqq = I, Fqv = dt I outside the floating-base blocks
+  auto kern_g = rbt::riccati_backward_kernel<INST_NV, INST_NU, INST_NS, NP, false>;  // any Fxx
   if (!h->attr_bwd) {  // the attribute is per device: tracked per handle (a handle lives on one device)
     RBT_CUDA(h, cudaFuncSetAttribute(kern_s, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES));
     RBT_CUDA(h, cudaFuncSetAttribute(kern_g, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES));
@@ -518,41 +530,35 @@ static int launch_backward(rbt_handle* h, int write_fact, cudaStream_t st) {
   }
   rbt::BwdParams p;
   p.L = h->L;
-  p.ctrl = h->d_ctrl;
-  const int b0 = win_b0(h), nb = win_nb(h);
-  const size_t go = size_t(b0) * h->n_grid;
+  p.ctrl = h->d_ctrl.get();
+  const size_t go = size_t(w.b0) * h->n_grid;
   p.n_grid = h->n_grid;
-  p.batch = nb;
+  p.batch = w.nb;
   p.max_dts0 = h->max_dts0;
-  p.kkt = h->d_kkt + go * h->L.k_stride;
-  p.ric = h->d_ric + go * h->L.r_stride;
-  p.fact = write_fact ? h->d_fact + go * h->L.f_stride : nullptr;
-  p.info = h->d_info + b0;
-  p.sm_arrivals = h->d_arrivals;
-  p.stagger_ns = h->stagger_ns;
-  p.timeline = h->d_timeline;
-  p.timeline_cta = h->timeline_cta;
+  p.kkt = h->buf[RBT_BUF_KKT] + go * h->L.k_stride;
+  p.ric = h->buf[RBT_BUF_RIC] + go * h->L.r_stride;
+  p.fact = write_fact ? h->buf[RBT_BUF_FACT] + go * h->L.f_stride : nullptr;
+  p.info = h->d_info.get() + w.b0;
   p.struct_flag = nullptr;
-  if (!h->keep_info) RBT_CUDA(h, cudaMemsetAsync(h->d_info + b0, 0, size_t(nb) * sizeof(int), st));
+  if (!h->keep_info) RBT_CUDA(h, cudaMemsetAsync(p.info, 0, size_t(w.nb) * sizeof(int), st));
   h->keep_info = false;
-  if (h->stagger_ns > 0) RBT_CUDA(h, cudaMemsetAsync(h->d_arrivals, 0, 1024 * sizeof(int), st));
   // Which instance: the condensing kernel writes Fqq = I, Fqv = dt I outside the floating-base blocks by construction
   // (state_equation.cpp:52-55,68-87), a caller can declare it (rbt_set_fxx_structure), otherwise (RBT_FXX_AUTO) the records are
   // inspected on the device and BOTH instances are launched -- the one the flag does not select returns at once.
   const bool known_struct = h->kkt_from_condense || h->fxx_mode == RBT_FXX_MECHANICAL;
   h->kkt_from_condense = false;
   if (known_struct) {
-    kern_s<<<nb, C::NTHREADS, C::SMEM_BYTES, st>>>(p);
+    kern_s<<<w.nb, C::NTHREADS, C::SMEM_BYTES, st>>>(p);
     h->launches += 1;
   } else if (h->fxx_mode == RBT_FXX_GENERAL) {
-    kern_g<<<nb, C::NTHREADS, C::SMEM_BYTES, st>>>(p);
+    kern_g<<<w.nb, C::NTHREADS, C::SMEM_BYTES, st>>>(p);
     h->launches += 1;
   } else {
-    RBT_CUDA(h, cudaMemsetAsync(h->d_struct, 0, 2 * sizeof(int), st));
-    rbt::check_fxx_structure_kernel<NV, NP><<<(nb * (h->n_grid - 1) + 7) / 8, 256, 0, st>>>(p, h->d_struct);
-    p.struct_flag = h->d_struct;
-    kern_s<<<nb, C::NTHREADS, C::SMEM_BYTES, st>>>(p);
-    kern_g<<<nb, C::NTHREADS, C::SMEM_BYTES, st>>>(p);
+    RBT_CUDA(h, cudaMemsetAsync(h->d_struct.get(), 0, 2 * sizeof(int), st));
+    rbt::check_fxx_structure_kernel<INST_NV, NP><<<(w.nb * (h->n_grid - 1) + 7) / 8, 256, 0, st>>>(p, h->d_struct.get());
+    p.struct_flag = h->d_struct.get();
+    kern_s<<<w.nb, C::NTHREADS, C::SMEM_BYTES, st>>>(p);
+    kern_g<<<w.nb, C::NTHREADS, C::SMEM_BYTES, st>>>(p);
     h->launches += 3;
   }
   RBT_CUDA(h, cudaGetLastError());
@@ -565,26 +571,24 @@ int rbt_set_fxx_structure(rbt_handle* h, int mode) {
   return RBT_OK;
 }
 
-template <int NV, int NU, int NS>
-static int launch_forward(rbt_handle* h, cudaStream_t st) {
-  using C = rbt::FwdCfg<NV, NU, NS>;
-  auto kern = rbt::riccati_forward_kernel<NV, NU, NS>;
+static int launch_forward(rbt_handle* h, Win w, cudaStream_t st) {
+  using C = rbt::FwdCfg<INST_NV, INST_NU, INST_NS>;
+  auto kern = rbt::riccati_forward_kernel<INST_NV, INST_NU, INST_NS>;
   if (!h->attr_fwd) {
     RBT_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES));
     h->attr_fwd = true;
   }
   rbt::FwdParams p;
   p.L = h->L;
-  p.ctrl = h->d_ctrl;
-  const int b0 = win_b0(h), nb = win_nb(h);
-  const size_t go = size_t(b0) * h->n_grid;
+  p.ctrl = h->d_ctrl.get();
+  const size_t go = size_t(w.b0) * h->n_grid;
   p.n_grid = h->n_grid;
-  p.batch = nb;
-  p.kkt = h->d_kkt + go * h->L.k_stride;
-  p.ric = h->d_ric + go * h->L.r_stride;
-  p.dx0 = h->d_dx0 + size_t(b0) * h->L.nx;
-  p.dir = h->d_dir + go * h->L.d_stride;
-  kern<<<nb, C::NTHREADS, C::SMEM_BYTES, st>>>(p);
+  p.batch = w.nb;
+  p.kkt = h->buf[RBT_BUF_KKT] + go * h->L.k_stride;
+  p.ric = h->buf[RBT_BUF_RIC] + go * h->L.r_stride;
+  p.dx0 = h->buf[RBT_BUF_DX0] + size_t(w.b0) * h->L.nx;
+  p.dir = h->buf[RBT_BUF_DIR] + go * h->L.d_stride;
+  kern<<<w.nb, C::NTHREADS, C::SMEM_BYTES, st>>>(p);
   RBT_CUDA(h, cudaGetLastError());
   h->launches += 1;
   return RBT_OK;
@@ -597,11 +601,7 @@ int rbt_riccati_backward(rbt_handle* h, int write_fact, void* stream) {
     return RBT_ERR_STATE;
   }
   RBT_CUDA(h, cudaSetDevice(h->device));
-#define X(NV, NU, NS) \
-  if (h->dims.nv == NV && h->dims.nu == NU && h->dims.ns_max == NS) return launch_backward<NV, NU, NS>(h, write_fact, (cudaStream_t)stream);
-  RBT_INSTANCES(X)
-#undef X
-  return RBT_ERR_ARG;
+  return launch_backward(h, {0, h->batch}, write_fact, (cudaStream_t)stream);
 }
 
 int rbt_riccati_forward(rbt_handle* h, void* stream) {
@@ -611,11 +611,7 @@ int rbt_riccati_forward(rbt_handle* h, void* stream) {
     return RBT_ERR_STATE;
   }
   RBT_CUDA(h, cudaSetDevice(h->device));
-#define X(NV, NU, NS) \
-  if (h->dims.nv == NV && h->dims.nu == NU && h->dims.ns_max == NS) return launch_forward<NV, NU, NS>(h, (cudaStream_t)stream);
-  RBT_INSTANCES(X)
-#undef X
-  return RBT_ERR_ARG;
+  return launch_forward(h, {0, h->batch}, (cudaStream_t)stream);
 }
 
 // ---- stage layer ---------------------------------------------------------------------------------------------------
@@ -659,7 +655,7 @@ int rbt_stage_setup(rbt_handle* h, const rbt_stage_dims* sd, const rbt_constrain
       }
     }
   }
-  if (h->stage_ready) {  // a second call would leak every stage buffer and leave stale own[] pointers behind a re-bound one
+  if (h->stage_ready) {  // a second call would replace stage buffers the caller may have re-bound
     h->err = "[rbt_stage_setup] already set up on this handle (create a new handle for another constraint table)";
     return RBT_ERR_STATE;
   }
@@ -673,7 +669,7 @@ int rbt_stage_setup(rbt_handle* h, const rbt_stage_dims* sd, const rbt_constrain
   h->stage_ready = false;
   rbt_make_stage_layout(sd, &h->S);
   {  // condense_kernel lands [l_D, l_Phix) and [l_ha, l_dgdq) of the record in place: the static mirror must match
-    using C = rbt::CondCfg<18, 12, 12>;
+    using C = rbt::CondCfg<INST_NV, INST_NU, INST_NS>;
     const rbt_stage_layout& S = h->S;
     const int gsz = (S.l_dgdf - S.l_dgdq) + ((15 * S.ncon + 1) & ~1);
     const int q0 = S.l_Quu - C::IN1A;  // record offset that maps onto the second in-place mirror
@@ -684,7 +680,7 @@ int rbt_stage_setup(rbt_handle* h, const rbt_stage_dims* sd, const rbt_constrain
                     S.l_hf - S.l_ha == C::j_hf && S.l_hx - S.l_ha == C::j_hx && S.l_hu - S.l_ha == C::j_hu &&
                     S.l_fx - S.l_ha == C::j_fx && S.l_sc - S.l_ha == C::j_sc &&
                     5 * S.ncp + gsz <= C::NVF * C::NX &&  // PDIPM staging fits in the R buffer
-                    S.l_J - S.l_M == rbt::MjtjCfg<18, 12>::o_J && S.l_D - S.l_M == rbt::MjtjCfg<18, 12>::MJ;
+                    S.l_J - S.l_M == rbt::MjtjCfg<INST_NV, INST_NU>::o_J && S.l_D - S.l_M == rbt::MjtjCfg<INST_NV, INST_NU>::MJ;
     if (!ok) {
       h->err = "[rbt_stage_setup] invalid argument: stage layout not supported by the compiled condensing kernel";
       return RBT_ERR_ARG;
@@ -695,17 +691,17 @@ int rbt_stage_setup(rbt_handle* h, const rbt_stage_dims* sd, const rbt_constrain
     return RBT_ERR_ARG;
   }
   RBT_CUDA(h, cudaSetDevice(h->device));
-  const size_t per = size_t(h->batch) * h->n_grid_max;
-  RBT_CUDA(h, cudaMalloc(&h->d_lin, per * h->S.l_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_con, per * h->S.c_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_ex, per * h->S.e_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_sol, per * h->S.s_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_xd, per * h->S.x_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_steps, size_t(h->batch) * 2 * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_ones, size_t(h->batch) * 2 * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_stage_perf, per * 4 * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_perf, size_t(h->batch) * 8 * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_x0in, size_t(h->batch) * 2 * h->dims.nv * 8));
+  // uploads skip record padding: the zeroed allocation keeps it defined
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_LIN, h->S.l_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_CON, h->S.c_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_EXP, h->S.e_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_SOL, h->S.s_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_XDIR, h->S.x_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_STEPS, 2, false));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_PERF, 8, false));
+  RBT_CUDA(h, dev_alloc(h->d_ones, size_t(h->batch) * 2));
+  RBT_CUDA(h, dev_alloc(h->d_stage_perf, size_t(h->batch) * h->n_grid_max * 4));
+  RBT_CUDA(h, dev_alloc(h->d_x0in, size_t(h->batch) * 2 * h->dims.nv));
   {  // box rows acting on each target entry (var, idx), in ascending row order (deterministic accumulation on the device):
      // entry = (row + 1) * sign, 0 = none.  Device memory, not kernel parameters: the lanes of a warp look up different targets,
      // and a divergent constant-bank access is serialised.
@@ -723,45 +719,74 @@ int rbt_stage_setup(rbt_handle* h, const rbt_stage_dims* sd, const rbt_constrain
     // point iff level + ineq_gate <= 2 (ConstraintsData::setTimeStage)
     int lvl[RBT_MAX_BOX_ROWS] = {};
     for (int r = 0; r < h->table.n_box; ++r) lvl[r] = h->table.box[r].var == RBT_VAR_Q ? 2 : (h->table.box[r].var == RBT_VAR_V ? 1 : 0);
-    RBT_CUDA(h, cudaMalloc(&h->d_tgt, sizeof(tg) + sizeof(lvl)));
-    RBT_CUDA(h, cudaMemcpy(h->d_tgt, tg, sizeof(tg), cudaMemcpyHostToDevice));
-    RBT_CUDA(h, cudaMemcpy(h->d_tgt + RBT_MAX_TARGETS * 4, lvl, sizeof(lvl), cudaMemcpyHostToDevice));
+    RBT_CUDA(h, dev_alloc(h->d_tgt, sizeof(tg) / sizeof(int) + sizeof(lvl) / sizeof(int)));
+    RBT_CUDA(h, cudaMemcpy(h->d_tgt.get(), tg, sizeof(tg), cudaMemcpyHostToDevice));
+    RBT_CUDA(h, cudaMemcpy(h->d_tgt.get() + RBT_MAX_TARGETS * 4, lvl, sizeof(lvl), cudaMemcpyHostToDevice));
   }
-  RBT_CUDA(h, cudaMemset(h->d_perf, 0, size_t(h->batch) * 8 * 8));
-  RBT_CUDA(h, cudaMemset(h->d_lin, 0, per * h->S.l_stride * 8));  // uploads skip record padding: keep it defined
-  RBT_CUDA(h, cudaMemset(h->d_sol, 0, per * h->S.s_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_ex, 0, per * h->S.e_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_xd, 0, per * h->S.x_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_con, 0, per * h->S.c_stride * 8));
   std::vector<double> ones(size_t(h->batch) * 2, 1.0);
-  RBT_CUDA(h, cudaMemcpy(h->d_ones, ones.data(), ones.size() * 8, cudaMemcpyHostToDevice));
-  RBT_CUDA(h, cudaMemcpy(h->d_steps, ones.data(), ones.size() * 8, cudaMemcpyHostToDevice));
+  RBT_CUDA(h, cudaMemcpy(h->d_ones.get(), ones.data(), ones.size() * 8, cudaMemcpyHostToDevice));
+  RBT_CUDA(h, cudaMemcpy(h->buf[RBT_BUF_STEPS], ones.data(), ones.size() * 8, cudaMemcpyHostToDevice));
   h->stage_ready = true;
   return RBT_OK;
 }
 
-static rbt::StageParams make_stage_params(rbt_handle* h) {
+static rbt::StageParams make_stage_params(rbt_handle* h, Win w) {
   rbt::StageParams p;
   p.K = h->L;
   p.S = h->S;
   p.tab = h->table;
-  p.ctrl = h->d_ctrl;
-  const int b0 = win_b0(h);
-  const size_t go = size_t(b0) * h->n_grid;
+  p.ctrl = h->d_ctrl.get();
+  const size_t go = size_t(w.b0) * h->n_grid;
   p.n_grid = h->n_grid;
-  p.batch = win_nb(h);
-  p.lin = h->d_lin + go * h->S.l_stride;
-  p.con = h->d_con + go * h->S.c_stride;
-  p.kkt = h->d_kkt + go * h->L.k_stride;
-  p.ex = h->d_ex + go * h->S.e_stride;
-  p.dir = h->d_dir + go * h->L.d_stride;
-  p.xd = h->d_xd + go * h->S.x_stride;
-  p.sol = h->d_sol + go * h->S.s_stride;
-  p.steps = h->d_steps + 2 * size_t(b0);
-  p.info = h->d_info + b0;
-  p.tgt = reinterpret_cast<const int4*>(h->d_tgt);
-  p.row_level = h->d_tgt + RBT_MAX_TARGETS * 4;
+  p.batch = w.nb;
+  p.lin = h->buf[RBT_BUF_LIN] + go * h->S.l_stride;
+  p.con = h->buf[RBT_BUF_CON] + go * h->S.c_stride;
+  p.kkt = h->buf[RBT_BUF_KKT] + go * h->L.k_stride;
+  p.ex = h->buf[RBT_BUF_EXP] + go * h->S.e_stride;
+  p.dir = h->buf[RBT_BUF_DIR] + go * h->L.d_stride;
+  p.xd = h->buf[RBT_BUF_XDIR] + go * h->S.x_stride;
+  p.sol = h->buf[RBT_BUF_SOL] + go * h->S.s_stride;
+  p.steps = h->buf[RBT_BUF_STEPS] + 2 * size_t(w.b0);
+  p.info = h->d_info.get() + w.b0;
+  p.tgt = reinterpret_cast<const int4*>(h->d_tgt.get());
+  p.row_level = h->d_tgt.get() + RBT_MAX_TARGETS * 4;
   return p;
+}
+
+static int launch_condense(rbt_handle* h, Win w, cudaStream_t st) {
+  using C = rbt::CondCfg<INST_NV, INST_NU, INST_NS>;
+  auto kern = rbt::condense_kernel<INST_NV, INST_NU, INST_NS>;
+  if (!h->attr_cond) {
+    RBT_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES));
+    h->attr_cond = true;
+  }
+  const rbt::StageParams p = make_stage_params(h, w);
+  RBT_CUDA(h, cudaMemsetAsync(p.info, 0, size_t(w.nb) * sizeof(int), st));
+  rbt::mjtjinv_kernel<INST_NV, INST_NU><<<(w.nb * h->n_grid + 1) / 2, 64, 0, st>>>(p);  // K1: Z = [[M,J^T],[J,0]]^-1
+  RBT_CUDA(h, cudaGetLastError());
+  if (h->ev_condense_mid) RBT_CUDA(h, cudaEventRecord(h->ev_condense_mid, st));
+  kern<<<w.nb * h->n_grid, C::NTHREADS, C::SMEM_BYTES, st>>>(p);                      // K2: condensing (DMMA)
+  RBT_CUDA(h, cudaGetLastError());
+  h->launches += 2;
+  h->keep_info = true;
+  h->kkt_from_condense = true;
+  return RBT_OK;
+}
+
+static int launch_expand(rbt_handle* h, Win w, cudaStream_t st) {
+  const rbt::StageParams p = make_stage_params(h, w);
+  RBT_CUDA(h, cudaMemcpyAsync(p.steps, h->d_ones.get(), size_t(w.nb) * 2 * 8, cudaMemcpyDeviceToDevice, st));
+  rbt::expand_kernel<INST_NV, INST_NU, INST_NS><<<w.nb * h->n_grid, rbt::XTHR, 0, st>>>(p);
+  RBT_CUDA(h, cudaGetLastError());
+  h->launches += 1;
+  return RBT_OK;
+}
+
+static int launch_update(rbt_handle* h, Win w, cudaStream_t st) {
+  rbt::update_kernel<INST_NV, INST_NU, INST_NS><<<w.nb * h->n_grid, rbt::XTHR, 0, st>>>(make_stage_params(h, w));
+  RBT_CUDA(h, cudaGetLastError());
+  h->launches += 1;
+  return RBT_OK;
 }
 
 #define RBT_STAGE_CHECK(h, what)                                  \
@@ -774,24 +799,7 @@ static rbt::StageParams make_stage_params(rbt_handle* h) {
 
 int rbt_condense(rbt_handle* h, void* stream) {
   RBT_STAGE_CHECK(h, "rbt_condense");
-  using C = rbt::CondCfg<18, 12, 12>;
-  auto kern = rbt::condense_kernel<18, 12, 12>;
-  if (!h->attr_cond) {
-    RBT_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES));
-    h->attr_cond = true;
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  const int nb = win_nb(h);
-  RBT_CUDA(h, cudaMemsetAsync(h->d_info + win_b0(h), 0, size_t(nb) * sizeof(int), st));
-  rbt::mjtjinv_kernel<18, 12><<<(nb * h->n_grid + 1) / 2, 64, 0, st>>>(make_stage_params(h));  // K1: Z = [[M,J^T],[J,0]]^-1
-  RBT_CUDA(h, cudaGetLastError());
-  if (h->ev_condense_mid) RBT_CUDA(h, cudaEventRecord(h->ev_condense_mid, st));
-  kern<<<nb * h->n_grid, C::NTHREADS, C::SMEM_BYTES, st>>>(make_stage_params(h));     // K2: condensing (DMMA)
-  RBT_CUDA(h, cudaGetLastError());
-  h->launches += 2;
-  h->keep_info = true;
-  h->kkt_from_condense = true;
-  return RBT_OK;
+  return launch_condense(h, {0, h->batch}, (cudaStream_t)stream);
 }
 
 int rbt_set_condense_event(rbt_handle* h, void* cuda_event) {
@@ -802,30 +810,22 @@ int rbt_set_condense_event(rbt_handle* h, void* cuda_event) {
 
 int rbt_expand_and_step_sizes(rbt_handle* h, void* stream) {
   RBT_STAGE_CHECK(h, "rbt_expand_and_step_sizes");
-  cudaStream_t st = (cudaStream_t)stream;
-  RBT_CUDA(h, cudaMemcpyAsync(h->d_steps + 2 * size_t(win_b0(h)), h->d_ones, size_t(win_nb(h)) * 2 * 8, cudaMemcpyDeviceToDevice, st));
-  rbt::expand_kernel<18, 12, 12><<<win_nb(h) * h->n_grid, rbt::XTHR, 0, st>>>(make_stage_params(h));
-  RBT_CUDA(h, cudaGetLastError());
-  h->launches += 1;
-  return RBT_OK;
+  return launch_expand(h, {0, h->batch}, (cudaStream_t)stream);
 }
 
 int rbt_update(rbt_handle* h, void* stream) {
   RBT_STAGE_CHECK(h, "rbt_update");
-  rbt::update_kernel<18, 12, 12><<<win_nb(h) * h->n_grid, rbt::XTHR, 0, (cudaStream_t)stream>>>(make_stage_params(h));
-  RBT_CUDA(h, cudaGetLastError());
-  h->launches += 1;
-  return RBT_OK;
+  return launch_update(h, {0, h->batch}, (cudaStream_t)stream);
 }
 
+// the whole batch
 static rbt::EvalParams make_eval_params(rbt_handle* h) {
   rbt::EvalParams q;
-  q.sp = make_stage_params(h);
-  const int b0 = win_b0(h);
-  q.stage_perf = h->d_stage_perf + size_t(b0) * h->n_grid * 4;
-  q.perf = h->d_perf + size_t(b0) * 8;
-  q.x0in = h->d_x0in + size_t(b0) * 2 * h->dims.nv;
-  q.dx0 = h->d_dx0 + size_t(b0) * h->L.nx;
+  q.sp = make_stage_params(h, {0, h->batch});
+  q.stage_perf = h->d_stage_perf.get();
+  q.perf = h->buf[RBT_BUF_PERF];
+  q.x0in = h->d_x0in.get();
+  q.dx0 = h->buf[RBT_BUF_DX0];
   return q;
 }
 
@@ -833,9 +833,8 @@ int rbt_eval_kkt(rbt_handle* h, void* stream) {
   RBT_STAGE_CHECK(h, "rbt_eval_kkt");
   cudaStream_t st = (cudaStream_t)stream;
   const rbt::EvalParams q = make_eval_params(h);
-  const int nb = win_nb(h);
-  rbt::perf_index_kernel<<<(nb * h->n_grid + 3) / 4, 128, 0, st>>>(q);
-  rbt::perf_reduce_kernel<<<(nb + 127) / 128, 128, 0, st>>>(q);
+  rbt::perf_index_kernel<<<(h->batch * h->n_grid + 3) / 4, 128, 0, st>>>(q);
+  rbt::perf_reduce_kernel<<<(h->batch + 127) / 128, 128, 0, st>>>(q);
   RBT_CUDA(h, cudaGetLastError());
   h->launches += 2;
   return RBT_OK;
@@ -844,7 +843,7 @@ int rbt_eval_kkt(rbt_handle* h, void* stream) {
 int rbt_set_slack_and_dual_positive(rbt_handle* h, void* stream) {
   RBT_STAGE_CHECK(h, "rbt_set_slack_and_dual_positive");
   const rbt::EvalParams q = make_eval_params(h);
-  const long long total = (long long)win_nb(h) * h->n_grid * h->S.ncp;
+  const long long total = (long long)h->batch * h->n_grid * h->S.ncp;
   rbt::slack_dual_positive_kernel<<<unsigned((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(q);
   RBT_CUDA(h, cudaGetLastError());
   h->launches += 1;
@@ -858,8 +857,8 @@ int rbt_set_joint_limits(rbt_handle* h, const double* bound_host) {
     return RBT_ERR_STATE;
   }
   RBT_CUDA(h, cudaSetDevice(h->device));
-  if (!h->d_bound) RBT_CUDA(h, cudaMalloc(&h->d_bound, sizeof(double) * RBT_MAX_BOX_ROWS));
-  RBT_CUDA(h, cudaMemcpy(h->d_bound, bound_host, sizeof(double) * h->table.n_box, cudaMemcpyHostToDevice));
+  if (!h->d_bound) RBT_CUDA(h, dev_alloc(h->d_bound, RBT_MAX_BOX_ROWS));
+  RBT_CUDA(h, cudaMemcpy(h->d_bound.get(), bound_host, sizeof(double) * h->table.n_box, cudaMemcpyHostToDevice));
   return RBT_OK;
 }
 
@@ -870,8 +869,8 @@ int rbt_linearize_joint_limits(rbt_handle* h, void* stream) {
     return RBT_ERR_STATE;
   }
   const rbt::EvalParams q = make_eval_params(h);
-  const long long total = (long long)win_nb(h) * h->n_grid * (3 * h->S.nv + h->S.nu);
-  rbt::linearize_joint_limits_kernel<<<unsigned((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(q, h->d_bound);
+  const long long total = (long long)h->batch * h->n_grid * (3 * h->S.nv + h->S.nu);
+  rbt::linearize_joint_limits_kernel<<<unsigned((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(q, h->d_bound.get());
   RBT_CUDA(h, cudaGetLastError());
   h->launches += 1;
   return RBT_OK;
@@ -881,9 +880,9 @@ int rbt_initial_state_direction(rbt_handle* h, const double* dq0_v0_host, void* 
   RBT_STAGE_CHECK(h, "rbt_initial_state_direction");
   if (!dq0_v0_host) return RBT_ERR_ARG;
   cudaStream_t st = (cudaStream_t)stream;
-  RBT_CUDA(h, cudaMemcpyAsync(h->d_x0in, dq0_v0_host, size_t(h->batch) * 2 * h->dims.nv * 8, cudaMemcpyHostToDevice, st));
+  RBT_CUDA(h, cudaMemcpyAsync(h->d_x0in.get(), dq0_v0_host, size_t(h->batch) * 2 * h->dims.nv * 8, cudaMemcpyHostToDevice, st));
   const rbt::EvalParams q = make_eval_params(h);
-  const int total = win_nb(h) * h->L.nx;
+  const int total = h->batch * h->L.nx;
   rbt::initial_state_direction_kernel<<<(total + 127) / 128, 128, 0, st>>>(q);
   RBT_CUDA(h, cudaGetLastError());
   h->launches += 1;
@@ -895,20 +894,18 @@ enum { RBT_LS_FILTER_CAP = 16 };
 
 static int ls_ensure(rbt_handle* h, int n_trials) {
   if (n_trials <= h->ls_trials) return RBT_OK;
-  cudaFree(h->d_ls_alphas); cudaFree(h->d_ls_trial); cudaFree(h->d_ls_stage_barrier); cudaFree(h->d_ls_barrier); cudaFree(h->d_ls_in);
-  h->d_ls_alphas = h->d_ls_trial = h->d_ls_stage_barrier = h->d_ls_barrier = h->d_ls_in = nullptr;
   const size_t kb = size_t(n_trials) * h->batch;
-  RBT_CUDA(h, cudaMalloc(&h->d_ls_alphas, kb * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_ls_barrier, kb * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_ls_stage_barrier, kb * h->n_grid_max * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_ls_trial, kb * h->n_grid_max * rbt::T_STRIDE * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_ls_in, (2 * kb + 2 * size_t(h->batch)) * 8));  // cost | viol of the trials, cost0 | viol0
+  RBT_CUDA(h, dev_alloc(h->d_ls_alphas, kb));
+  RBT_CUDA(h, dev_alloc(h->d_ls_barrier, kb));
+  RBT_CUDA(h, dev_alloc(h->d_ls_stage_barrier, kb * h->n_grid_max));
+  RBT_CUDA(h, dev_alloc(h->d_ls_trial, kb * h->n_grid_max * rbt::T_STRIDE));
+  RBT_CUDA(h, dev_alloc(h->d_ls_in, 2 * kb + 2 * size_t(h->batch)));  // cost | viol of the trials, cost0 | viol0
   if (!h->d_ls_filt) {
-    RBT_CUDA(h, cudaMalloc(&h->d_ls_filt, size_t(h->batch) * 2 * RBT_LS_FILTER_CAP * 8));
-    RBT_CUDA(h, cudaMalloc(&h->d_ls_nfilt, size_t(h->batch) * sizeof(int)));
-    RBT_CUDA(h, cudaMalloc(&h->d_ls_step, size_t(h->batch) * 8));
-    RBT_CUDA(h, cudaMalloc(&h->d_ls_k, size_t(h->batch) * sizeof(int)));
-    RBT_CUDA(h, cudaMemset(h->d_ls_nfilt, 0, size_t(h->batch) * sizeof(int)));
+    RBT_CUDA(h, dev_alloc(h->d_ls_filt, size_t(h->batch) * 2 * RBT_LS_FILTER_CAP));
+    RBT_CUDA(h, dev_alloc(h->d_ls_nfilt, h->batch));
+    RBT_CUDA(h, dev_alloc(h->d_ls_step, h->batch));
+    RBT_CUDA(h, dev_alloc(h->d_ls_k, h->batch));
+    RBT_CUDA(h, cudaMemset(h->d_ls_nfilt.get(), 0, size_t(h->batch) * sizeof(int)));
   }
   h->ls_trials = n_trials;
   return RBT_OK;
@@ -926,30 +923,30 @@ int rbt_line_search_trials(rbt_handle* h, int n_trials, double step_size_reducti
   if (int rc = ls_ensure(h, n_trials)) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   rbt::TrialParams q;
-  q.sp = make_stage_params(h);
+  q.sp = make_stage_params(h, {0, h->batch});
   q.n_trials = n_trials;
   q.rate = step_size_reduction_rate;
-  q.alphas = h->d_ls_alphas;
-  q.trial = h->d_ls_trial;
-  q.stage_barrier = h->d_ls_stage_barrier;
-  q.barrier = h->d_ls_barrier;
+  q.alphas = h->d_ls_alphas.get();
+  q.trial = h->d_ls_trial.get();
+  q.stage_barrier = h->d_ls_stage_barrier.get();
+  q.barrier = h->d_ls_barrier.get();
   const long long warps = (long long)n_trials * h->batch * h->n_grid;
   rbt::trial_solution_kernel<<<unsigned((warps + 3) / 4), 128, 0, st>>>(q);
   rbt::trial_reduce_kernel<<<(n_trials * h->batch + 127) / 128, 128, 0, st>>>(q);
   RBT_CUDA(h, cudaGetLastError());
   h->launches += 2;
   const size_t kb = size_t(n_trials) * h->batch;
-  if (alphas_host) RBT_CUDA(h, cudaMemcpyAsync(alphas_host, h->d_ls_alphas, kb * 8, cudaMemcpyDeviceToHost, st));
-  if (barrier_host) RBT_CUDA(h, cudaMemcpyAsync(barrier_host, h->d_ls_barrier, kb * 8, cudaMemcpyDeviceToHost, st));
-  if (trial_host) RBT_CUDA(h, cudaMemcpyAsync(trial_host, h->d_ls_trial, kb * h->n_grid * rbt::T_STRIDE * 8, cudaMemcpyDeviceToHost, st));
+  if (alphas_host) RBT_CUDA(h, cudaMemcpyAsync(alphas_host, h->d_ls_alphas.get(), kb * 8, cudaMemcpyDeviceToHost, st));
+  if (barrier_host) RBT_CUDA(h, cudaMemcpyAsync(barrier_host, h->d_ls_barrier.get(), kb * 8, cudaMemcpyDeviceToHost, st));
+  if (trial_host) RBT_CUDA(h, cudaMemcpyAsync(trial_host, h->d_ls_trial.get(), kb * h->n_grid * rbt::T_STRIDE * 8, cudaMemcpyDeviceToHost, st));
   return RBT_OK;
 }
 
-double* rbt_line_search_trial_dev(rbt_handle* h) { return h ? h->d_ls_trial : nullptr; }
+double* rbt_line_search_trial_dev(rbt_handle* h) { return h ? h->d_ls_trial.get() : nullptr; }
 
 int rbt_line_search_clear_history(rbt_handle* h, void* stream) {
   if (!h) return RBT_ERR_ARG;
-  if (h->d_ls_nfilt) RBT_CUDA(h, cudaMemsetAsync(h->d_ls_nfilt, 0, size_t(h->batch) * sizeof(int), (cudaStream_t)stream));
+  if (h->d_ls_nfilt) RBT_CUDA(h, cudaMemsetAsync(h->d_ls_nfilt.get(), 0, size_t(h->batch) * sizeof(int), (cudaStream_t)stream));
   return RBT_OK;
 }
 
@@ -966,9 +963,9 @@ int rbt_line_search_filter(rbt_handle* h, int n_trials, double step_size_reducti
   }
   cudaStream_t st = (cudaStream_t)stream;
   const size_t kb = size_t(n_trials) * h->batch;
-  double* d_cost = h->d_ls_in;
-  double* d_viol = h->d_ls_in + size_t(h->ls_trials) * h->batch;
-  double* d_c0 = h->d_ls_in + 2 * size_t(h->ls_trials) * h->batch;
+  double* d_cost = h->d_ls_in.get();
+  double* d_viol = d_cost + size_t(h->ls_trials) * h->batch;
+  double* d_c0 = d_cost + 2 * size_t(h->ls_trials) * h->batch;
   double* d_v0 = d_c0 + h->batch;
   RBT_CUDA(h, cudaMemcpyAsync(d_cost, cost_host, kb * 8, cudaMemcpyHostToDevice, st));
   RBT_CUDA(h, cudaMemcpyAsync(d_viol, violation_host, kb * 8, cudaMemcpyHostToDevice, st));
@@ -978,112 +975,39 @@ int rbt_line_search_filter(rbt_handle* h, int n_trials, double step_size_reducti
   q.batch = h->batch; q.n_trials = n_trials; q.cap = RBT_LS_FILTER_CAP;
   q.rate = step_size_reduction_rate; q.min_step = min_step_size;
   q.cost_rate = filter_cost_reduction_rate; q.viol_rate = filter_constraint_violation_reduction_rate;
-  q.steps = h->d_steps; q.cost0 = d_c0; q.viol0 = d_v0; q.cost = d_cost; q.barrier = h->d_ls_barrier; q.viol = d_viol;
-  q.filt = h->d_ls_filt; q.nfilt = h->d_ls_nfilt; q.out_step = h->d_ls_step; q.out_k = h->d_ls_k;
+  q.steps = h->buf[RBT_BUF_STEPS]; q.cost0 = d_c0; q.viol0 = d_v0; q.cost = d_cost; q.barrier = h->d_ls_barrier.get(); q.viol = d_viol;
+  q.filt = h->d_ls_filt.get(); q.nfilt = h->d_ls_nfilt.get(); q.out_step = h->d_ls_step.get(); q.out_k = h->d_ls_k.get();
   rbt::line_search_filter_kernel<<<(h->batch + 127) / 128, 128, 0, st>>>(q);
   RBT_CUDA(h, cudaGetLastError());
   h->launches += 1;
-  if (step_host) RBT_CUDA(h, cudaMemcpyAsync(step_host, h->d_ls_step, size_t(h->batch) * 8, cudaMemcpyDeviceToHost, st));
-  if (accepted_trial_host) RBT_CUDA(h, cudaMemcpyAsync(accepted_trial_host, h->d_ls_k, size_t(h->batch) * sizeof(int), cudaMemcpyDeviceToHost, st));
+  if (step_host) RBT_CUDA(h, cudaMemcpyAsync(step_host, h->d_ls_step.get(), size_t(h->batch) * 8, cudaMemcpyDeviceToHost, st));
+  if (accepted_trial_host) RBT_CUDA(h, cudaMemcpyAsync(accepted_trial_host, h->d_ls_k.get(), size_t(h->batch) * sizeof(int), cudaMemcpyDeviceToHost, st));
   return RBT_OK;
 }
 
-// Host <-> device traffic of the stage layer, for the batch window [b0, b0 + nb).  Only what the kernels read / what
-// persists crosses PCIe: record padding never does, the switching-constraint section of the linearization record only for
-// the stages that carry one, of the PDIPM record slack | dual | residual go up and slack | dual come back.
-static long long stage_xfer(rbt_handle* h, int which, bool up, const double* host_c, double* host_m, int b0, int nb,
-                            cudaStream_t st, bool do_copy, int* rc_out) {
-  const rbt_stage_layout& S = h->S;
-  const size_t rows = size_t(nb) * h->n_grid, go = size_t(b0) * h->n_grid;
-  long long bytes = 0;
-  auto copy2d = [&](double* dev, const double* hc, double* hm, size_t off, size_t stride, size_t width, size_t pitch_rows,
-                    size_t nrows) {
-    bytes += (long long)(width * 8 * nrows);
-    if (!do_copy || *rc_out != RBT_OK) return;
-    const size_t pitch = stride * pitch_rows * 8;
-    if (pitch == width * 8) {  // contiguous: one linear DMA
-      cudaError_t e1 = up ? cudaMemcpyAsync(dev + off, hc + off, width * 8 * nrows, cudaMemcpyHostToDevice, st)
-                          : cudaMemcpyAsync(hm + off, dev + off, width * 8 * nrows, cudaMemcpyDeviceToHost, st);
-      if (e1 != cudaSuccess) *rc_out = RBT_ERR_CUDA;
-      return;
-    }
-    cudaError_t e = up ? cudaMemcpy2DAsync(dev + off, pitch, hc + off, pitch, width * 8, nrows, cudaMemcpyHostToDevice, st)
-                       : cudaMemcpy2DAsync(hm + off, pitch, dev + off, pitch, width * 8, nrows, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) *rc_out = RBT_ERR_CUDA;
-  };
-  if (which == RBT_XFER_WIRE) {  // packed wire records: contiguous
-    copy2d(h->d_wire, host_c, host_m, size_t(b0) * h->w_ocp, h->w_ocp, h->w_ocp, 1, nb);
-  } else if (which == RBT_XFER_SWITCHING) {  // only the switching-constraint sections of the classic record
-    const size_t base = go * S.l_stride;
-    for (int i = 0; i < h->n_grid; ++i)
-      if (h->ctrl[i].ns > 0 && h->ctrl[i].type != RBT_IMPACT)
-        copy2d(h->d_lin, host_c, host_m, base + size_t(i) * S.l_stride + S.l_Phix, S.l_stride, S.l_ha - S.l_Phix, h->n_grid, nb);
-  } else if (which == RBT_BUF_LIN) {
-    const size_t base = go * S.l_stride;
-    const size_t tail = size_t(S.l_dgdf) + ((15 * S.ncon + 1) & ~1) - S.l_ha;
-    copy2d(h->d_lin, host_c, host_m, base, S.l_stride, S.l_Phix, 1, rows);            // M .. se3
-    copy2d(h->d_lin, host_c, host_m, base + S.l_ha, S.l_stride, tail, 1, rows);       // ha .. dgdf
-    for (int i = 0; i < h->n_grid; ++i)
-      if (h->ctrl[i].ns > 0 && h->ctrl[i].type != RBT_IMPACT)                         // Phix, Phia, p, Phit
-        copy2d(h->d_lin, host_c, host_m, base + size_t(i) * S.l_stride + S.l_Phix, S.l_stride, S.l_ha - S.l_Phix, h->n_grid, nb);
-  } else if (which == RBT_XFER_RES) {  // compact PDIPM residuals [batch][n_grid][ncp]: one contiguous copy into the staging buffer
-    copy2d(h->d_res_stage, host_c, host_m, go * S.ncp, S.ncp, S.ncp, 1, rows);   // (unpack_wire_kernel scatters them into c_res)
-  } else if (which == RBT_XFER_SD) {   // compact slack | dual [batch][n_grid][2 ncp] (packed by pack_slack_dual_kernel): contiguous
-    copy2d(h->d_sd_stage, host_c, host_m, go * 2 * S.ncp, 2 * S.ncp, 2 * S.ncp, 1, rows);
-
-  } else if (which == RBT_BUF_CON) {
-    copy2d(h->d_con, host_c, host_m, go * S.c_stride + S.c_slack, S.c_stride, size_t(up ? 3 : 2) * S.ncp, 1, rows);
-  } else if (which == RBT_BUF_SOL) {
-    // whole records incl. the few padding doubles: ONE contiguous DMA instead of a strided 2-D copy of 1.4 KB rows (the copy
-    // engine spends as long per row as on ~4 KB of payload)
-    copy2d(h->d_sol, host_c, host_m, go * S.s_stride, S.s_stride, S.s_stride, 1, rows);
-  } else if (which == RBT_BUF_DX0) {
-    copy2d(h->d_dx0, host_c, host_m, size_t(b0) * h->L.nx, h->L.nx, h->L.nx, 1, nb);
-  } else if (which == RBT_BUF_STEPS) {
-    copy2d(h->d_steps, host_c, host_m, 2 * size_t(b0), 2, 2, 1, nb);
-  }
-  return bytes;
-}
-
-int rbt_iteration_host_bytes(rbt_handle* h, int wire, long long* h2d, long long* d2h) {
+int rbt_iteration_host_bytes(rbt_handle* h, int mode, long long* h2d, long long* d2h) {
   if (!h || !h->stage_ready || h->n_grid == 0) return RBT_ERR_STATE;
-  int rc = RBT_OK;
-  long long up = 0, down = 0;
-  h->w_ocp = make_wire_layouts(h->S, h->ctrl.data(), h->n_grid, h->cost_structure, h->Wv);
-  if (wire == 2) {  // rbt_iteration_host_resident: wire records + residuals + dx0 up
-    up += stage_xfer(h, RBT_XFER_WIRE, true, nullptr, nullptr, 0, h->batch, nullptr, false, &rc);
-    up += stage_xfer(h, RBT_XFER_SWITCHING, true, nullptr, nullptr, 0, h->batch, nullptr, false, &rc);
-    up += stage_xfer(h, RBT_XFER_RES, true, nullptr, nullptr, 0, h->batch, nullptr, false, &rc);
-    up += stage_xfer(h, RBT_BUF_DX0, true, nullptr, nullptr, 0, h->batch, nullptr, false, &rc);
-    for (int w : {int(RBT_BUF_SOL), int(RBT_XFER_SD), int(RBT_BUF_STEPS)}) down += stage_xfer(h, w, false, nullptr, nullptr, 0, h->batch, nullptr, false, &rc);
-    if (h2d) *h2d = up;
-    if (d2h) *d2h = down;
-    return RBT_OK;
+  if (mode != DENSE && mode != WIRE && mode != RESIDENT) return RBT_ERR_ARG;
+  if (mode != DENSE) {
+    RBT_CUDA(h, cudaSetDevice(h->device));
+    if (int rc = ensure_wire_layouts(h)) return rc;
   }
-  if (wire) {
-    up += stage_xfer(h, RBT_XFER_WIRE, true, nullptr, nullptr, 0, h->batch, nullptr, false, &rc);
-    up += stage_xfer(h, RBT_XFER_SWITCHING, true, nullptr, nullptr, 0, h->batch, nullptr, false, &rc);
-  } else {
-    up += stage_xfer(h, RBT_BUF_LIN, true, nullptr, nullptr, 0, h->batch, nullptr, false, &rc);
-  }
-  for (int w : {RBT_BUF_CON, RBT_BUF_SOL, RBT_BUF_DX0}) up += stage_xfer(h, w, true, nullptr, nullptr, 0, h->batch, nullptr, false, &rc);
-  for (int w : {RBT_BUF_SOL, RBT_BUF_CON, RBT_BUF_STEPS}) down += stage_xfer(h, w, false, nullptr, nullptr, 0, h->batch, nullptr, false, &rc);
-  if (h2d) *h2d = up;
-  if (d2h) *d2h = down;
+  const std::vector<Copy> plan = host_plan(h, HostMode(mode), {0, h->batch});
+  if (h2d) *h2d = plan_bytes(plan, cudaMemcpyHostToDevice);
+  if (d2h) *d2h = plan_bytes(plan, cudaMemcpyDeviceToHost);
   return RBT_OK;
 }
 
-// res_host != NULL: resident mode (solution, slack and dual stay where the previous iteration left them on the device; only the
-// PDIPM residuals come from the host), con_host / sol_host are not read.
-static int iteration_host_impl(rbt_handle* h, const double* wire_host, const double* lin_host, const double* con_host,
-                               const double* sol_host, const double* res_host, const double* dx0_host, double* sol_out,
-                               double* con_out, double* steps_out, void* stream) {
-  if (!h || (!lin_host && !wire_host) || !dx0_host) return RBT_ERR_ARG;
-  if (!res_host && (!con_host || !sol_host)) return RBT_ERR_ARG;
+// RESIDENT: solution, slack and dual stay where the previous iteration left them on the device; only the PDIPM residuals
+// come from the host, con_host / sol_host are not read.  WIRE, RESIDENT: lin_host holds the switching-constraint sections.
+static int iteration_host_impl(rbt_handle* h, HostMode mode, const double* wire_host, const double* lin_host,
+                               const double* con_host, const double* sol_host, const double* res_host, const double* dx0_host,
+                               double* sol_out, double* con_out, double* steps_out, void* stream) {
+  if (!h || (mode == DENSE ? !lin_host : !wire_host) || !dx0_host) return RBT_ERR_ARG;
+  if (mode == RESIDENT ? !res_host : (!con_host || !sol_host)) return RBT_ERR_ARG;
   RBT_STAGE_CHECK(h, "rbt_iteration_host");
-  if (wire_host) {
-    int rcw = ensure_wire_layouts(h);
-    if (rcw != RBT_OK) return rcw;
+  if (mode != DENSE) {
+    if (int rc = ensure_wire_layouts(h)) return rc;
     bool sw = false;
     for (int i = 0; i < h->n_grid; ++i) sw = sw || (h->ctrl[i].ns > 0 && h->ctrl[i].type != RBT_IMPACT);
     if (sw && !lin_host) {
@@ -1095,113 +1019,102 @@ static int iteration_host_impl(rbt_handle* h, const double* wire_host, const dou
       rbt_stage_ctrl cmax = {};
       cmax.type = RBT_INTERMEDIATE; cmax.nf = h->S.nfm; cmax.contact_mask = (1 << h->S.ncon) - 1;
       rbt_make_wire_layout(&h->S, &cmax, 1, RBT_COST_GENERAL, &wmax);
-      RBT_CUDA(h, cudaMalloc(&h->d_wire, size_t(h->batch) * h->n_grid_max * wmax.w_doubles * 8));
-    }
-    if (res_host && !h->d_res_stage) {
-      RBT_CUDA(h, cudaMalloc(&h->d_res_stage, size_t(h->batch) * h->n_grid_max * h->S.ncp * 8));
-      RBT_CUDA(h, cudaMalloc(&h->d_sd_stage, size_t(h->batch) * h->n_grid_max * 2 * h->S.ncp * 8));
+      RBT_CUDA(h, dev_alloc(h->d_wire, size_t(h->batch) * h->n_grid_max * wmax.w_doubles));
     }
   }
+  if (mode == RESIDENT && !h->d_res_stage) {
+    RBT_CUDA(h, dev_alloc(h->d_res_stage, size_t(h->batch) * h->n_grid_max * h->S.ncp));
+    RBT_CUDA(h, dev_alloc(h->d_sd_stage, size_t(h->batch) * h->n_grid_max * 2 * h->S.ncp));
+  }
+  const double* in[N_HOST_ARGS] = {};
+  double* out[N_HOST_ARGS] = {};
+  in[A_WIRE] = wire_host, in[A_LIN] = lin_host, in[A_CON] = con_host, in[A_SOL] = sol_host, in[A_RES] = res_host;
+  in[A_DX0] = dx0_host;
+  out[A_SOL_OUT] = sol_out, out[A_CON_OUT] = con_out, out[A_STEPS_OUT] = steps_out;
   cudaStream_t st = (cudaStream_t)stream;
   // chunks of the batch: the upload of chunk c+1, the kernels of chunk c and the download of chunk c-1 overlap
   int n_chunks = h->batch >= 512 ? 8 : (h->batch >= 128 ? 4 : 1);
   if (const char* e = getenv("RBT_E2E_CHUNKS")) n_chunks = std::max(1, std::min(atoi(e), h->batch));
   if (!h->s_h2d) {
-    RBT_CUDA(h, cudaStreamCreateWithFlags(&h->s_h2d, cudaStreamNonBlocking));
-    RBT_CUDA(h, cudaStreamCreateWithFlags(&h->s_d2h, cudaStreamNonBlocking));
+    cudaStream_t s1, s2;
+    RBT_CUDA(h, cudaStreamCreateWithFlags(&s1, cudaStreamNonBlocking));
+    h->s_h2d.reset(s1);
+    RBT_CUDA(h, cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking));
+    h->s_d2h.reset(s2);
   }
   while ((int)h->ev.size() < 2 * n_chunks + 2) {
     cudaEvent_t e;
     RBT_CUDA(h, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    h->ev.push_back(e);
+    h->ev.emplace_back(e);
   }
-  cudaEvent_t ev_entry = h->ev[2 * n_chunks], ev_exit = h->ev[2 * n_chunks + 1];
+  cudaStream_t s_h2d = h->s_h2d.get(), s_d2h = h->s_d2h.get();
+  cudaEvent_t ev_entry = h->ev[2 * n_chunks].get(), ev_exit = h->ev[2 * n_chunks + 1].get();
   RBT_CUDA(h, cudaEventRecord(ev_entry, st));            // device buffers may still be read by earlier work on `stream`
-  RBT_CUDA(h, cudaStreamWaitEvent(h->s_h2d, ev_entry, 0));
-  RBT_CUDA(h, cudaStreamWaitEvent(h->s_d2h, ev_entry, 0));
-  int rc = RBT_OK;
-  for (int c = 0; c < n_chunks && rc == RBT_OK; ++c) {
-    const int b0 = int((long long)h->batch * c / n_chunks), b1 = int((long long)h->batch * (c + 1) / n_chunks), nb = b1 - b0;
-    if (nb <= 0) continue;
-    if (wire_host) {
-      stage_xfer(h, RBT_XFER_WIRE, true, wire_host, nullptr, b0, nb, h->s_h2d, true, &rc);
-      if (lin_host) stage_xfer(h, RBT_XFER_SWITCHING, true, lin_host, nullptr, b0, nb, h->s_h2d, true, &rc);
-    } else {
-      stage_xfer(h, RBT_BUF_LIN, true, lin_host, nullptr, b0, nb, h->s_h2d, true, &rc);
-    }
-    if (res_host) {
-      stage_xfer(h, RBT_XFER_RES, true, res_host, nullptr, b0, nb, h->s_h2d, true, &rc);
-    } else {
-      stage_xfer(h, RBT_BUF_CON, true, con_host, nullptr, b0, nb, h->s_h2d, true, &rc);
-      stage_xfer(h, RBT_BUF_SOL, true, sol_host, nullptr, b0, nb, h->s_h2d, true, &rc);
-    }
-    stage_xfer(h, RBT_BUF_DX0, true, dx0_host, nullptr, b0, nb, h->s_h2d, true, &rc);
-    if (rc != RBT_OK) break;
-    RBT_CUDA(h, cudaEventRecord(h->ev[2 * c], h->s_h2d));
-    RBT_CUDA(h, cudaStreamWaitEvent(st, h->ev[2 * c], 0));
-    h->cb0 = b0;
-    h->cnb = nb;
-    if (wire_host) {  // expand the packed records of this chunk into the linearization records
+  RBT_CUDA(h, cudaStreamWaitEvent(s_h2d, ev_entry, 0));
+  RBT_CUDA(h, cudaStreamWaitEvent(s_d2h, ev_entry, 0));
+  for (int c = 0; c < n_chunks; ++c) {
+    const int b0 = int((long long)h->batch * c / n_chunks), b1 = int((long long)h->batch * (c + 1) / n_chunks);
+    const Win w{b0, b1 - b0};
+    if (w.nb <= 0) continue;
+    const std::vector<Copy> plan = host_plan(h, mode, w);
+    for (const Copy& k : plan)
+      if (k.kind == cudaMemcpyHostToDevice && in[k.arg])
+        if (int rc = issue(h, k, in[k.arg], nullptr, s_h2d)) return rc;
+    cudaEvent_t ev_up = h->ev[2 * c].get(), ev_done = h->ev[2 * c + 1].get();
+    RBT_CUDA(h, cudaEventRecord(ev_up, s_h2d));
+    RBT_CUDA(h, cudaStreamWaitEvent(st, ev_up, 0));
+    const size_t go = size_t(b0) * h->n_grid;
+    if (mode != DENSE) {  // expand the packed records of this chunk into the linearization records
       rbt::WireParams wp;
-      wp.W = h->d_W;
+      wp.W = h->d_W.get();
       wp.n_grid = h->n_grid;
       wp.ocp_stride = h->w_ocp;
       wp.l_stride = h->S.l_stride;
-      wp.wire = h->d_wire + size_t(b0) * h->w_ocp;
-      wp.lin = h->d_lin + size_t(b0) * h->n_grid * h->S.l_stride;
-      wp.res = res_host ? h->d_res_stage + size_t(b0) * h->n_grid * h->S.ncp : nullptr;
-      wp.con = h->d_con + size_t(b0) * h->n_grid * h->S.c_stride;
+      wp.wire = h->d_wire.get() + size_t(b0) * h->w_ocp;
+      wp.lin = h->buf[RBT_BUF_LIN] + go * h->S.l_stride;
+      wp.res = mode == RESIDENT ? h->d_res_stage.get() + go * h->S.ncp : nullptr;
+      wp.con = h->buf[RBT_BUF_CON] + go * h->S.c_stride;
       wp.c_stride = h->S.c_stride; wp.c_res = h->S.c_res; wp.ncp = h->S.ncp;
-      rbt::unpack_wire_kernel<<<nb * h->n_grid, 128, 0, st>>>(wp);
+      rbt::unpack_wire_kernel<<<w.nb * h->n_grid, 128, 0, st>>>(wp);
       h->launches += 1;
     }
-    if (!(rc = rbt_condense(h, stream)) && !(rc = rbt_riccati_backward(h, 0, stream)) && !(rc = rbt_riccati_forward(h, stream)) &&
-        !(rc = rbt_expand_and_step_sizes(h, stream)))
-      rc = rbt_update(h, stream);
-    h->cb0 = 0;
-    h->cnb = 0;
-    if (rc != RBT_OK) break;
-    if (res_host && con_out) {
-      rbt::pack_slack_dual_kernel<<<nb * h->n_grid, 64, 0, st>>>(h->d_con + size_t(b0) * h->n_grid * h->S.c_stride, h->S.c_stride,
-                                                               h->S.c_slack, 2 * h->S.ncp,
-                                                               h->d_sd_stage + size_t(b0) * h->n_grid * 2 * h->S.ncp);
+    int rc;
+    if ((rc = launch_condense(h, w, st)) || (rc = launch_backward(h, w, 0, st)) || (rc = launch_forward(h, w, st)) ||
+        (rc = launch_expand(h, w, st)) || (rc = launch_update(h, w, st)))
+      return rc;
+    if (mode == RESIDENT && con_out) {
+      rbt::pack_slack_dual_kernel<<<w.nb * h->n_grid, 64, 0, st>>>(h->buf[RBT_BUF_CON] + go * h->S.c_stride, h->S.c_stride,
+                                                                 h->S.c_slack, 2 * h->S.ncp, h->d_sd_stage.get() + go * 2 * h->S.ncp);
       h->launches += 1;
     }
-    RBT_CUDA(h, cudaEventRecord(h->ev[2 * c + 1], st));
-    RBT_CUDA(h, cudaStreamWaitEvent(h->s_d2h, h->ev[2 * c + 1], 0));
-    if (sol_out) stage_xfer(h, RBT_BUF_SOL, false, nullptr, sol_out, b0, nb, h->s_d2h, true, &rc);
-    if (con_out) stage_xfer(h, res_host ? RBT_XFER_SD : RBT_BUF_CON, false, nullptr, con_out, b0, nb, h->s_d2h, true, &rc);
-    if (steps_out) stage_xfer(h, RBT_BUF_STEPS, false, nullptr, steps_out, b0, nb, h->s_d2h, true, &rc);
+    RBT_CUDA(h, cudaEventRecord(ev_done, st));
+    RBT_CUDA(h, cudaStreamWaitEvent(s_d2h, ev_done, 0));
+    for (const Copy& k : plan)
+      if (k.kind == cudaMemcpyDeviceToHost && out[k.arg])
+        if (int rc2 = issue(h, k, nullptr, out[k.arg], s_d2h)) return rc2;
   }
-  h->cb0 = 0;
-  h->cnb = 0;
-  if (rc != RBT_OK) {
-    if (h->err.empty() || rc == RBT_ERR_CUDA) h->err = std::string("rbt_iteration_host: ") + cudaGetErrorString(cudaGetLastError());
-    return rc;
-  }
-  RBT_CUDA(h, cudaEventRecord(ev_exit, h->s_d2h));       // `stream` (what the caller synchronizes) covers the downloads too
+  RBT_CUDA(h, cudaEventRecord(ev_exit, s_d2h));       // `stream` (what the caller synchronizes) covers the downloads too
   RBT_CUDA(h, cudaStreamWaitEvent(st, ev_exit, 0));
   return RBT_OK;
 }
 
 int rbt_iteration_host(rbt_handle* h, const double* lin_host, const double* con_host, const double* sol_host,
                        const double* dx0_host, double* sol_out, double* con_out, double* steps_out, void* stream) {
-  if (!lin_host) return RBT_ERR_ARG;
-  return iteration_host_impl(h, nullptr, lin_host, con_host, sol_host, nullptr, dx0_host, sol_out, con_out, steps_out, stream);
+  return iteration_host_impl(h, DENSE, nullptr, lin_host, con_host, sol_host, nullptr, dx0_host, sol_out, con_out, steps_out,
+                             stream);
 }
 
 int rbt_iteration_host_wire(rbt_handle* h, const double* wire_host, const double* lin_host_switching, const double* con_host,
                             const double* sol_host, const double* dx0_host, double* sol_out, double* con_out,
                             double* steps_out, void* stream) {
-  if (!wire_host || !con_host || !sol_host) return RBT_ERR_ARG;
-  return iteration_host_impl(h, wire_host, lin_host_switching, con_host, sol_host, nullptr, dx0_host, sol_out, con_out, steps_out, stream);
+  return iteration_host_impl(h, WIRE, wire_host, lin_host_switching, con_host, sol_host, nullptr, dx0_host, sol_out, con_out,
+                             steps_out, stream);
 }
 
 int rbt_iteration_host_resident(rbt_handle* h, const double* wire_host, const double* lin_host_switching, const double* res_host,
                                 const double* dx0_host, double* sol_out, double* slack_dual_out, double* steps_out, void* stream) {
-  if (!wire_host || !res_host) return RBT_ERR_ARG;
-  return iteration_host_impl(h, wire_host, lin_host_switching, nullptr, nullptr, res_host, dx0_host, sol_out, slack_dual_out, steps_out,
-                             stream);
+  return iteration_host_impl(h, RESIDENT, wire_host, lin_host_switching, nullptr, nullptr, res_host, dx0_host, sol_out,
+                             slack_dual_out, steps_out, stream);
 }
 
 int rbt_set_wire_cost_structure(rbt_handle* h, int cost_structure) {
@@ -1294,7 +1207,7 @@ int rbt_pack_step(rbt_handle* h, double* packed_dev, void* stream) {
   RBT_CUDA(h, cudaSetDevice(h->device));
   const int step = h->L.d_dts + 2;
   const long long n_rec = (long long)h->batch * h->n_grid;
-  pack_step_kernel<<<unsigned((n_rec * step + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->d_dir, packed_dev, h->L.d_stride, step, n_rec);
+  pack_step_kernel<<<unsigned((n_rec * step + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->buf[RBT_BUF_DIR], packed_dev, h->L.d_stride, step, n_rec);
   RBT_CUDA(h, cudaGetLastError());
   h->launches += 1;
   return RBT_OK;
@@ -1312,9 +1225,9 @@ int rbt_allgather_step(rbt_handle* h, void* nccl_comm, double* all_dev, void* st
   cudaStream_t st = (cudaStream_t)stream;
   const int step = h->L.d_dts + 2;
   const long long n_rec = (long long)h->batch * h->n_grid;
-  if (!h->d_step_pack) RBT_CUDA(h, cudaMalloc(&h->d_step_pack, size_t(h->batch) * h->n_grid_max * step * 8));
-  if (int prc = rbt_pack_step(h, h->d_step_pack, stream)) return prc;
-  const int rc = allgather(h->d_step_pack, all_dev, size_t(n_rec) * step, /*ncclFloat64*/ 8, nccl_comm, st);
+  if (!h->d_step_pack) RBT_CUDA(h, dev_alloc(h->d_step_pack, size_t(h->batch) * h->n_grid_max * step));
+  if (int prc = rbt_pack_step(h, h->d_step_pack.get(), stream)) return prc;
+  const int rc = allgather(h->d_step_pack.get(), all_dev, size_t(n_rec) * step, /*ncclFloat64*/ 8, nccl_comm, st);
   if (rc != 0) {
     h->err = "[rbt_allgather_step] ncclAllGather failed with ncclResult_t " + std::to_string(rc);
     return RBT_ERR_CUDA;
@@ -1331,129 +1244,63 @@ int rbt_sync(rbt_handle* h, void* stream) {
 
 const char* rbt_last_error(rbt_handle* h) { return h ? h->err.c_str() : "null handle"; }
 
-// bring-up only (not part of the public header): copy the timeline stamps of the last backward launch
-extern "C" int rbt_debug_timeline(rbt_handle* h, long long* host, int n) {
-  if (!h || !h->d_timeline) return RBT_ERR_STATE;
-  return cudaMemcpy(host, h->d_timeline, size_t(n) * sizeof(long long), cudaMemcpyDeviceToHost) == cudaSuccess ? RBT_OK : RBT_ERR_CUDA;
-}
 long long rbt_launch_count(rbt_handle* h) { return h ? h->launches : 0; }
 
 // ---------------------------------------------------------------------------------------------------------------
 // unconstrained path
 // ---------------------------------------------------------------------------------------------------------------
-#define RBT_UINSTANCES(X) X(7)
-
 int rbt_unconstr_create(int nv, int N, double dt, int batch, int device, rbt_uhandle** out) {
-  if (!out || nv < 1 || N < 1 || batch < 1 || !(dt > 0)) return RBT_ERR_ARG;
-  bool ok = false;
-#define X(NV) \
-  if (nv == NV) ok = true;
-  RBT_UINSTANCES(X)
-#undef X
-  if (!ok) return RBT_ERR_ARG;
+  if (!out || nv != UINST_NV || N < 1 || batch < 1 || !(dt > 0)) return RBT_ERR_ARG;
   rbt_uhandle* h = new rbt_uhandle();
   h->nv = nv;
   h->N = N;
   h->dt = dt;
   h->batch = batch;
   h->device = device;
+  h->buf.batch = batch;
+  h->buf.n_grid_max = N + 1;
   rbt_make_ulayout(nv, &h->L);
   *out = h;
   RBT_CUDA(h, cudaSetDevice(device));
-  const size_t per = size_t(batch) * (N + 1);
-  RBT_CUDA(h, cudaMalloc(&h->d_kkt, per * h->L.k_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_ric, per * h->L.r_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_fact, per * h->L.f_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_dir, per * h->L.d_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_dx0, size_t(batch) * h->L.nx * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_info, size_t(batch) * sizeof(int)));
-  RBT_CUDA(h, cudaMemset(h->d_ric, 0, per * h->L.r_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_fact, 0, per * h->L.f_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_dir, 0, per * h->L.d_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_info, 0, size_t(batch) * sizeof(int)));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_KKT, h->L.k_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_RIC, h->L.r_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_FACT, h->L.f_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_DIR, h->L.d_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_DX0, h->L.nx, false));
+  RBT_CUDA(h, dev_alloc(h->d_info, batch));
+  RBT_CUDA(h, cudaMemset(h->d_info.get(), 0, size_t(batch) * sizeof(int)));
   return RBT_OK;
 }
 
 int rbt_unconstr_destroy(rbt_uhandle* h) {
   if (!h) return RBT_ERR_ARG;
   cudaSetDevice(h->device);
-  cudaFree(h->d_kkt);
-  cudaFree(h->d_ric);
-  cudaFree(h->d_fact);
-  cudaFree(h->d_dir);
-  cudaFree(h->d_dx0);
-  cudaFree(h->d_info);
-  cudaFree(h->d_lin);
-  cudaFree(h->d_con);
-  cudaFree(h->d_ex);
-  cudaFree(h->d_sol);
-  cudaFree(h->d_xd);
-  cudaFree(h->d_steps);
-  cudaFree(h->d_ones);
   delete h;
   return RBT_OK;
 }
 
-static double* ubuf_ptr(rbt_uhandle* h, int which) {
-  switch (which) {
-    case RBT_BUF_KKT: return h->d_kkt;
-    case RBT_BUF_RIC: return h->d_ric;
-    case RBT_BUF_FACT: return h->d_fact;
-    case RBT_BUF_DIR: return h->d_dir;
-    case RBT_BUF_DX0: return h->d_dx0;
-    case RBT_BUF_LIN: return h->d_lin;
-    case RBT_BUF_CON: return h->d_con;
-    case RBT_BUF_EXP: return h->d_ex;
-    case RBT_BUF_SOL: return h->d_sol;
-    case RBT_BUF_XDIR: return h->d_xd;
-    case RBT_BUF_STEPS: return h->d_steps;
-    default: return nullptr;
-  }
-}
+long long rbt_unconstr_buf_doubles(rbt_uhandle* h, int which) { return h ? h->buf.doubles(which, h->N + 1) : -1; }
 
-long long rbt_unconstr_buf_doubles(rbt_uhandle* h, int which) {
-  if (!h) return -1;
-  const long long per = (long long)h->batch * (h->N + 1);
-  switch (which) {
-    case RBT_BUF_KKT: return per * h->L.k_stride;
-    case RBT_BUF_RIC: return per * h->L.r_stride;
-    case RBT_BUF_FACT: return per * h->L.f_stride;
-    case RBT_BUF_DIR: return per * h->L.d_stride;
-    case RBT_BUF_DX0: return (long long)h->batch * h->L.nx;
-    default: break;
-  }
-  if (!h->stage_ready) return -1;
-  switch (which) {
-    case RBT_BUF_LIN: return per * h->S.l_stride;
-    case RBT_BUF_CON: return per * h->S.c_stride;
-    case RBT_BUF_EXP: return per * h->S.e_stride;
-    case RBT_BUF_SOL: return per * h->S.s_stride;
-    case RBT_BUF_XDIR: return per * h->S.x_stride;
-    case RBT_BUF_STEPS: return (long long)h->batch * 2;
-    default: return -1;
-  }
-}
-
-double* rbt_unconstr_dev_ptr(rbt_uhandle* h, int which) { return h ? ubuf_ptr(h, which) : nullptr; }
+double* rbt_unconstr_dev_ptr(rbt_uhandle* h, int which) { return h ? h->buf[which] : nullptr; }
 
 int rbt_unconstr_upload(rbt_uhandle* h, int which, const double* host, void* stream) {
   if (!h || !host) return RBT_ERR_ARG;
   if (which != RBT_BUF_KKT && which != RBT_BUF_DX0 && which != RBT_BUF_LIN && which != RBT_BUF_CON && which != RBT_BUF_SOL)
     return RBT_ERR_ARG;
-  if (!ubuf_ptr(h, which)) {
+  if (!h->buf[which]) {
     h->err = "rbt_unconstr_upload: stage layer not set up (rbt_unconstr_stage_setup)";
     return RBT_ERR_STATE;
   }
   RBT_CUDA(h, cudaSetDevice(h->device));
-  RBT_CUDA(h, cudaMemcpyAsync(ubuf_ptr(h, which), host, size_t(rbt_unconstr_buf_doubles(h, which)) * 8,
+  RBT_CUDA(h, cudaMemcpyAsync(h->buf[which], host, size_t(rbt_unconstr_buf_doubles(h, which)) * 8,
                               cudaMemcpyHostToDevice, (cudaStream_t)stream));
   return RBT_OK;
 }
 
 int rbt_unconstr_download(rbt_uhandle* h, int which, double* host, void* stream) {
-  if (!h || !host || !ubuf_ptr(h, which)) return RBT_ERR_ARG;
+  if (!h || !host || !h->buf[which]) return RBT_ERR_ARG;
   RBT_CUDA(h, cudaSetDevice(h->device));
-  RBT_CUDA(h, cudaMemcpyAsync(host, ubuf_ptr(h, which), size_t(rbt_unconstr_buf_doubles(h, which)) * 8,
+  RBT_CUDA(h, cudaMemcpyAsync(host, h->buf[which], size_t(rbt_unconstr_buf_doubles(h, which)) * 8,
                               cudaMemcpyDeviceToHost, (cudaStream_t)stream));
   return RBT_OK;
 }
@@ -1461,24 +1308,23 @@ int rbt_unconstr_download(rbt_uhandle* h, int which, double* host, void* stream)
 int rbt_unconstr_download_info(rbt_uhandle* h, int* host_flags, void* stream) {
   if (!h || !host_flags) return RBT_ERR_ARG;
   RBT_CUDA(h, cudaSetDevice(h->device));
-  RBT_CUDA(h, cudaMemcpyAsync(host_flags, h->d_info, size_t(h->batch) * sizeof(int), cudaMemcpyDeviceToHost,
+  RBT_CUDA(h, cudaMemcpyAsync(host_flags, h->d_info.get(), size_t(h->batch) * sizeof(int), cudaMemcpyDeviceToHost,
                               (cudaStream_t)stream));
   return RBT_OK;
 }
 
-template <int NV>
 static rbt::UParams make_uparams(rbt_uhandle* h, int write_fact) {
   rbt::UParams p;
   p.L = h->L;
   p.N = h->N;
   p.batch = h->batch;
   p.dt = h->dt;
-  p.kkt = h->d_kkt;
-  p.ric = h->d_ric;
-  p.fact = write_fact ? h->d_fact : nullptr;
-  p.dx0 = h->d_dx0;
-  p.dir = h->d_dir;
-  p.info = h->d_info;
+  p.kkt = h->buf[RBT_BUF_KKT];
+  p.ric = h->buf[RBT_BUF_RIC];
+  p.fact = write_fact ? h->buf[RBT_BUF_FACT] : nullptr;
+  p.dx0 = h->buf[RBT_BUF_DX0];
+  p.dir = h->buf[RBT_BUF_DIR];
+  p.info = h->d_info.get();
   return p;
 }
 
@@ -1486,34 +1332,21 @@ int rbt_unconstr_backward(rbt_uhandle* h, int write_fact, void* stream) {
   if (!h) return RBT_ERR_ARG;
   RBT_CUDA(h, cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;
-#define X(NV)                                                                                  \
-  if (h->nv == NV) {                                                                           \
-    if (rbt::UCfg<NV>::KSTRIDE != h->L.k_stride) return RBT_ERR_STATE;                          \
-    RBT_CUDA(h, cudaMemsetAsync(h->d_info, 0, size_t(h->batch) * sizeof(int), st));            \
-    rbt::unconstr_backward_kernel<NV><<<h->batch, 32, 0, st>>>(make_uparams<NV>(h, write_fact)); \
-    RBT_CUDA(h, cudaGetLastError());                                                           \
-    h->launches += 1;                                                                          \
-    return RBT_OK;                                                                             \
-  }
-  RBT_UINSTANCES(X)
-#undef X
-  return RBT_ERR_ARG;
+  if (rbt::UCfg<UINST_NV>::KSTRIDE != h->L.k_stride) return RBT_ERR_STATE;
+  RBT_CUDA(h, cudaMemsetAsync(h->d_info.get(), 0, size_t(h->batch) * sizeof(int), st));
+  rbt::unconstr_backward_kernel<UINST_NV><<<h->batch, 32, 0, st>>>(make_uparams(h, write_fact));
+  RBT_CUDA(h, cudaGetLastError());
+  h->launches += 1;
+  return RBT_OK;
 }
 
 int rbt_unconstr_forward(rbt_uhandle* h, void* stream) {
   if (!h) return RBT_ERR_ARG;
   RBT_CUDA(h, cudaSetDevice(h->device));
-  cudaStream_t st = (cudaStream_t)stream;
-#define X(NV)                                                                         \
-  if (h->nv == NV) {                                                                  \
-    rbt::unconstr_forward_kernel<NV><<<h->batch, 32, 0, st>>>(make_uparams<NV>(h, 0)); \
-    RBT_CUDA(h, cudaGetLastError());                                                  \
-    h->launches += 1;                                                                 \
-    return RBT_OK;                                                                    \
-  }
-  RBT_UINSTANCES(X)
-#undef X
-  return RBT_ERR_ARG;
+  rbt::unconstr_forward_kernel<UINST_NV><<<h->batch, 32, 0, (cudaStream_t)stream>>>(make_uparams(h, 0));
+  RBT_CUDA(h, cudaGetLastError());
+  h->launches += 1;
+  return RBT_OK;
 }
 
 int rbt_unconstr_solve_host(rbt_uhandle* h, const double* kkt_host, const double* dx0_host, double* ric_host,
@@ -1565,22 +1398,16 @@ int rbt_unconstr_stage_setup(rbt_uhandle* h, const rbt_constraint_table* table) 
   RBT_CUDA(h, cudaSetDevice(h->device));
   rbt_make_ustage_layout(h->nv, table->n_box, &h->S);
   h->table = *table;
-  const size_t per = size_t(h->batch) * (h->N + 1);
-  RBT_CUDA(h, cudaMalloc(&h->d_lin, per * h->S.l_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_con, per * h->S.c_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_ex, per * h->S.e_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_sol, per * h->S.s_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_xd, per * h->S.x_stride * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_steps, size_t(h->batch) * 2 * 8));
-  RBT_CUDA(h, cudaMalloc(&h->d_ones, size_t(h->batch) * 2 * 8));
-  RBT_CUDA(h, cudaMemset(h->d_lin, 0, per * h->S.l_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_con, 0, per * h->S.c_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_ex, 0, per * h->S.e_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_sol, 0, per * h->S.s_stride * 8));
-  RBT_CUDA(h, cudaMemset(h->d_xd, 0, per * h->S.x_stride * 8));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_LIN, h->S.l_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_CON, h->S.c_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_EXP, h->S.e_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_SOL, h->S.s_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_XDIR, h->S.x_stride, true));
+  RBT_CUDA(h, h->buf.alloc(RBT_BUF_STEPS, 2, false));
+  RBT_CUDA(h, dev_alloc(h->d_ones, size_t(h->batch) * 2));
   std::vector<double> ones(size_t(h->batch) * 2, 1.0);
-  RBT_CUDA(h, cudaMemcpy(h->d_ones, ones.data(), ones.size() * 8, cudaMemcpyHostToDevice));
-  RBT_CUDA(h, cudaMemcpy(h->d_steps, ones.data(), ones.size() * 8, cudaMemcpyHostToDevice));
+  RBT_CUDA(h, cudaMemcpy(h->d_ones.get(), ones.data(), ones.size() * 8, cudaMemcpyHostToDevice));
+  RBT_CUDA(h, cudaMemcpy(h->buf[RBT_BUF_STEPS], ones.data(), ones.size() * 8, cudaMemcpyHostToDevice));
   h->stage_ready = true;
   return RBT_OK;
 }
@@ -1593,14 +1420,14 @@ static rbt::UStageParams make_ustage_params(rbt_uhandle* h) {
   p.N = h->N;
   p.batch = h->batch;
   p.dt = h->dt;
-  p.lin = h->d_lin;
-  p.con = h->d_con;
-  p.kkt = h->d_kkt;
-  p.ex = h->d_ex;
-  p.dir = h->d_dir;
-  p.xd = h->d_xd;
-  p.sol = h->d_sol;
-  p.steps = h->d_steps;
+  p.lin = h->buf[RBT_BUF_LIN];
+  p.con = h->buf[RBT_BUF_CON];
+  p.kkt = h->buf[RBT_BUF_KKT];
+  p.ex = h->buf[RBT_BUF_EXP];
+  p.dir = h->buf[RBT_BUF_DIR];
+  p.xd = h->buf[RBT_BUF_XDIR];
+  p.sol = h->buf[RBT_BUF_SOL];
+  p.steps = h->buf[RBT_BUF_STEPS];
   return p;
 }
 
@@ -1616,49 +1443,31 @@ static rbt::UStageParams make_ustage_params(rbt_uhandle* h) {
 int rbt_unconstr_condense(rbt_uhandle* h, void* stream) {
   RBT_USTAGE_GUARD(h)
   const size_t total = size_t(h->batch) * (h->N + 1);
-#define X(NV)                                                                                         \
-  if (h->nv == NV) {                                                                                  \
-    if (rbt::UStageCfg<NV>::LSTRIDE != h->S.l_stride) return RBT_ERR_STATE;                            \
-    constexpr int W = rbt::UStageCfg<NV>::WARPS;                                                      \
-    rbt::ucondense_kernel<NV><<<unsigned((total + W - 1) / W), 32 * W, 0, st>>>(make_ustage_params(h)); \
-    RBT_CUDA(h, cudaGetLastError());                                                                  \
-    h->launches += 1;                                                                                 \
-    return RBT_OK;                                                                                    \
-  }
-  RBT_UINSTANCES(X)
-#undef X
-  return RBT_ERR_ARG;
+  if (rbt::UStageCfg<UINST_NV>::LSTRIDE != h->S.l_stride) return RBT_ERR_STATE;
+  constexpr int W = rbt::UStageCfg<UINST_NV>::WARPS;
+  rbt::ucondense_kernel<UINST_NV><<<unsigned((total + W - 1) / W), 32 * W, 0, st>>>(make_ustage_params(h));
+  RBT_CUDA(h, cudaGetLastError());
+  h->launches += 1;
+  return RBT_OK;
 }
 
 int rbt_unconstr_expand_and_step_sizes(rbt_uhandle* h, void* stream) {
   RBT_USTAGE_GUARD(h)
   const size_t total = size_t(h->batch) * h->N;
-  RBT_CUDA(h, cudaMemcpyAsync(h->d_steps, h->d_ones, size_t(h->batch) * 2 * 8, cudaMemcpyDeviceToDevice, st));
-#define X(NV)                                                                                 \
-  if (h->nv == NV) {                                                                          \
-    rbt::uexpand_kernel<NV><<<unsigned((total + 3) / 4), 128, 0, st>>>(make_ustage_params(h)); \
-    RBT_CUDA(h, cudaGetLastError());                                                          \
-    h->launches += 1;                                                                         \
-    return RBT_OK;                                                                            \
-  }
-  RBT_UINSTANCES(X)
-#undef X
-  return RBT_ERR_ARG;
+  RBT_CUDA(h, cudaMemcpyAsync(h->buf[RBT_BUF_STEPS], h->d_ones.get(), size_t(h->batch) * 2 * 8, cudaMemcpyDeviceToDevice, st));
+  rbt::uexpand_kernel<UINST_NV><<<unsigned((total + 3) / 4), 128, 0, st>>>(make_ustage_params(h));
+  RBT_CUDA(h, cudaGetLastError());
+  h->launches += 1;
+  return RBT_OK;
 }
 
 int rbt_unconstr_update(rbt_uhandle* h, void* stream) {
   RBT_USTAGE_GUARD(h)
   const size_t total = size_t(h->batch) * (h->N + 1);
-#define X(NV)                                                                                 \
-  if (h->nv == NV) {                                                                          \
-    rbt::uupdate_kernel<NV><<<unsigned((total + 3) / 4), 128, 0, st>>>(make_ustage_params(h)); \
-    RBT_CUDA(h, cudaGetLastError());                                                          \
-    h->launches += 1;                                                                         \
-    return RBT_OK;                                                                            \
-  }
-  RBT_UINSTANCES(X)
-#undef X
-  return RBT_ERR_ARG;
+  rbt::uupdate_kernel<UINST_NV><<<unsigned((total + 3) / 4), 128, 0, st>>>(make_ustage_params(h));
+  RBT_CUDA(h, cudaGetLastError());
+  h->launches += 1;
+  return RBT_OK;
 }
 
 int rbt_unconstr_iteration_host(rbt_uhandle* h, const double* lin_host, const double* con_host, const double* sol_host,

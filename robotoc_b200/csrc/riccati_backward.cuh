@@ -38,11 +38,7 @@ struct BwdParams {
   double* ric;        // [batch][n_grid][r_stride]
   double* fact;       // [batch][n_grid][f_stride] or nullptr
   int* info;          // [batch]
-  int* sm_arrivals;   // [>= #SMs], zeroed before the launch (CTA de-phasing)
-  int stagger_ns;     // delay unit between co-resident CTAs (0 = off)
   const int* struct_flag;  // device: 0 = every Fxx of the batch has the mechanical structure (nullptr: run unconditionally)
-  long long* timeline;  // bring-up: [n_grid][2 roles][16] clock64 stamps of CTA `timeline_cta` (nullptr = off)
-  int timeline_cta;
 };
 
 // NP = dim_passive (6: floating base, 0: fixed base).  STRUCT: the state-equation blocks have the structure every robotoc
@@ -223,11 +219,6 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
   double* sc = vec + C::v_sc;
 
   int bad = 0;  // Cholesky failure flags (thread-local, OR-reduced at the end)
-  const bool tl_on = p.timeline != nullptr && b == p.timeline_cta && lane == 0 && (warp == 0 || !gemm_warp);
-#define RBT_TL(stage, slot)                                                                  \
-  do {                                                                                       \
-    if (tl_on) p.timeline[(size_t(stage) * 2 + (gemm_warp ? 0 : 1)) * 16 + (slot)] = clock64(); \
-  } while (0)
 
   auto issue_stage_load = [&](int st) {
     // one elected thread: stage st's [Fxx|Fvu|Fx|lx|lu] (+ extras when flagged)
@@ -248,14 +239,6 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
     mbar_init(&bars[0], 1);
     mbar_init(&bars[1], 1);
     fence_mbar_init();
-    // De-phase the CTAs that share an SM: they execute identical stage programs, so without an offset they all hit
-    // the tensor pipe together and then all sit in their latency-bound tails together.
-    if (p.stagger_ns > 0) {
-      unsigned smid;
-      asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-      const int rank = atomicAdd(&p.sm_arrivals[smid], 1) & 3;
-      for (int q = 0; q < rank; ++q) __nanosleep(p.stagger_ns);
-    }
   }
   __syncthreads();
   if (tid == 0 && N > 0) issue_stage_load(N - 1);
@@ -373,14 +356,12 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
     }
 
     // ---- wait for this stage's blocks
-    RBT_TL(i, 0);
     mbar_wait(&bars[0], par0);
     par0 ^= 1;
     if (extras) {
       mbar_wait(&bars[1], par1);
       par1 ^= 1;
     }
-    RBT_TL(i, 1);
 
     if (gemm_warp) {
       // ================= phase A (GEMM warps): Bp = Bv^T P+_vv (for the factor warp) ; AtP = A^T P+ ; z = s+ - P+ Fx
@@ -428,7 +409,6 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
           if (mine) *reinterpret_cast<double2*>(&sAtP[(i0 + g) * NX + j0 + 2 * t]) = make_double2(acc[n][0], acc[n][1]);
         }
       }
-      RBT_TL(i, 2);
       // Qxx -> accumulator fragments of F: issued here so the loads fly during z, but are not live across GEMM1
 #pragma unroll
       for (int n = 0; n < TX; ++n) {
@@ -455,7 +435,6 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
       }
       __syncwarp();  // this warp's rows of AtP are all the next two products read of it ...
       if (NX % 8 != 0 && warp >= TX - 2) named_bar_sync(5, 64);  // ... plus, for the last band, the rows the band before it stored
-      RBT_TL(i, 3);
 
       // ================= phase B (GEMM warps): F = Qxx + AtP A ; H = Qxu + AtP[:,nv:] Bv
       if constexpr (STRUCT) {
@@ -478,7 +457,6 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
         warp_mma_band<NX, TX, NX, false>(
             cF, i0, [&](int ii, int k) { return sAtP[ii * NX + k]; }, [&](int k, int j) { return sA[k + j * NX]; }, nb0);
       }
-      RBT_TL(i, 4);
       if (!impact) {
         warp_mma_band<NV, TU, NU, false>(
             cH, i0, [&](int ii, int k) { return sAtP[ii * NX + NV + k]; }, [&](int k, int u) { return sB[k + u * NV]; });
@@ -497,7 +475,6 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
           }
         }
       }
-      RBT_TL(i, 5);
       named_bar_sync(1, NG);  // z (and, for the STO terms, every row of AtP) complete among the GEMM warps
       if (!impact) {
         // lu' = lu - Bv^T z_v      (== lu + BtP Fx - Bv^T s+_v, backward_..factorizer.cpp:43-44)
@@ -508,7 +485,6 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
         });
       }
       matvec_T(sA, NX, NX, NX, z, tid, NG, [&](int c, double a) { t1[c] = a - slx[c]; });
-      RBT_TL(i, 6);
       if (sto) {
         if (!impact) {
           // factorizeHamiltonian (x part): backward_riccati_recursion_factorizer.cpp:48-66; the same lane owns psix[c]
@@ -528,7 +504,6 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
       // ================= factor warp: G = Quu + (Bv^T P+_vv) Bv, then L (G = L L^T) and L^-1 in registers
       if (!impact) {
         named_bar_sync(3, NTHR);  // Bp = Bv^T P+[nv:, nv:] from the GEMM warps
-        RBT_TL(i, 2);
 #pragma unroll
         for (int ub = 0; ub < TU; ++ub) {  // G = Quu + Bp Bv
           const int u0 = tile_off(ub, NU);
@@ -546,7 +521,6 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
           }
         }
         __syncwarp();
-        RBT_TL(i, 3);
         if (plain) {
           // Cholesky factor (rows on lanes 0..NU-1) and its inverse (columns on lanes 16..16+NU-1), broadcasts by shuffle
           double gc[NU], rs;
@@ -568,13 +542,10 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
           }
           __syncwarp();
         }
-        RBT_TL(i, 4);
       }
     }
-    RBT_TL(i, 7);
     if (tid == 0) tma_store_wait_read();  // the previous stage's bulk store of P has long read shared memory (issued ~3 us ago)
     __syncthreads();  // ---- barrier 2: AtP/H/t1 (GEMM warps) and G = L L^T, lu' (factor warp) are complete
-    RBT_TL(i, 8);
 
     // staging buffer is dead on plain stages: prefetch the next stage now (overlaps the rest of the stage)
     const bool early_prefetch = !extras;
@@ -626,9 +597,7 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
           for (int k = 0; k < NU; ++k) a = fma(sLi[lane + k * NU], lu2[k], a);
           ylu[lane] = a;
         }
-        RBT_TL(i, 9);
         __syncthreads();  // ---- barrier 3: Y complete
-        RBT_TL(i, 10);
         // ================= phase D
         if (gemm_warp) {
           // F -= Y^T Y
@@ -887,9 +856,7 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
         }
       }
     }
-    RBT_TL(i, 11);
     __syncthreads();  // ---- barrier 4: P (or the F scratch), s, k complete
-    RBT_TL(i, 12);
 
     if (fastP) {
       if (tid == 0) {
@@ -981,9 +948,7 @@ __global__ void __launch_bounds__(BwdCfg<NV, NU, NS, NP>::NTHREADS, RBT_BWD_MIN_
       }
       if (tid < 8) scn[tid] = 0.0;
     }
-    RBT_TL(i, 13);
     __syncthreads();  // ---- barrier 5: P+ / s+ / STO state rolled
-    RBT_TL(i, 14);
     if (!early_prefetch && tid == 0 && i > 0) issue_stage_load(i - 1);
   }
 
